@@ -6,7 +6,7 @@ random-spheres, 1200x800, 10 spp, depth 50) — every sample's camera ray genera
 traversal + intersection and scatter/shade, i.e. everything under Renderer::render
 (reference src/renderer.rs:42-105) except the PPM write.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1] [--impl reference] [--dump-outputs DIR]
 
 The one JSON line carries, next to the headline (`value`, C1 device-timed):
   parity    the framebuffer of the TIMED configuration against the CPU oracle on the same Philox stream
@@ -19,6 +19,9 @@ N > 1 (launched by torch.distributed.run): sample-range sharding.  `value` is we
 renders `spp_per_gpu` samples per pixel of its own absolute sample range over the full image (the image
 then has N x spp_per_gpu samples; `config.spp` says so), one framebuffer reduce over NCCL at the end; no
 collective inside the wavefront loop.
+
+--dump-outputs DIR writes the last timed step's output as .npy files (see dump_outputs) so that two builds can be
+compared output for output: the inputs depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -35,8 +38,13 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+# the benchmark leaves the tree as build() left it (it may be read-only): it imports modules build() does not
+# (scenes, meshes, distributed), and their bytecode caches would otherwise be written next to the sources
+sys.dont_write_bytecode = True
 
 METRIC = "Mrays/s"
+DUMP_BYTES = 64 << 20     # --dump-outputs: at most this much in all
+DUMP_SAMPLE_PIXELS = 1 << 21   # 40 MB with their indices
 
 
 # --------------------------------------------------------------------------------------------
@@ -260,6 +268,25 @@ def _claim_stdout():
     return real
 
 
+def dump_outputs(out_dir, image, counts):
+    """What the timed path returned in its last step: ``framebuffer.npy``, the (H, W, 3) float32 raw per-pixel sums
+    (RENDER_RAW_SUM, reduced over the ranks), and ``counts.npy``, float64 [rays, samples] of that step over all ranks.
+    An image larger than DUMP_BYTES is written as a fixed, seeded sample of its pixels instead:
+    ``framebuffer_sample.npy`` (n, 3) and ``framebuffer_sample_index.npy``, their row-major pixel indices (float64).
+    The counts repeat exactly from run to run; the sums only to a few float32 ulps, since the samples of a pixel are
+    added in the order their paths finish."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "counts.npy", np.asarray(counts, np.float64))
+    if image.nbytes + 4096 <= DUMP_BYTES:     # (room for the .npy headers and counts.npy)
+        np.save(out / "framebuffer.npy", image)
+        return
+    n_px = image.shape[0] * image.shape[1]
+    idx = np.sort(np.random.default_rng(0).choice(n_px, min(n_px, DUMP_SAMPLE_PIXELS), replace=False))
+    np.save(out / "framebuffer_sample.npy", image.reshape(n_px, 3)[idx])
+    np.save(out / "framebuffer_sample_index.npy", idx.astype(np.float64))
+
+
 def load_ncu():
     """ncu figures per config (thread instructions per ray, active lanes, issue utilisation, DRAM bytes) measured once
     per kernel change under gpurun and committed under profiles/ (tools/ncu_summary.py writes the file)."""
@@ -454,6 +481,12 @@ def main_gpu(args):
         flush.zero_()  # L2 flush between timed steps (outside the event pair)
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs:
+        counts = torch.tensor([float(stats[-1].rays), float(stats[-1].samples)], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, image_sum.cpu().numpy(), counts.cpu().numpy())
     # roofline pass: the same step again with CUDA events around every launch of the closest-hit kernel (on its stream)
     prof_stats = []
     for _ in range(args.profile_steps):
@@ -645,7 +678,13 @@ def main():
     ap.add_argument("--extra-cpu-s", type=float, default=5.0)
     ap.add_argument("--strong-spp", type=int, default=160)
     ap.add_argument("--strong-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's framebuffer and ray / sample counts as .npy files under DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,7 +1,7 @@
 """Generates rust/shimmer-patch/shimmer-b200.patch: the changes to the reference crate (a checkout of
-jalberse/RayTracingInOneWeekendInRust, /root/reference here) that route Renderer::render through libshimmer_b200.
+jalberse/RayTracingInOneWeekendInRust) that route Renderer::render through libshimmer_b200.
 
-    python rust/shimmer-patch/make_patch.py [/root/reference]
+    python rust/shimmer-patch/make_patch.py REFERENCE_CHECKOUT [OUT]     (OUT: the committed patch by default)
 
 It copies Cargo.toml and src/ of the reference to a temporary tree, applies the edits below, adds src/backend.rs
 (rust/shimmer-patch/backend.rs) and writes the unified diff (-U2, paths a/ b/: apply with `patch -p1` or `git apply`).
@@ -15,7 +15,6 @@ import tempfile
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-REF = Path(sys.argv[1] if len(sys.argv) > 1 else "/root/reference")
 
 REC_T = "    fn record(&self, r: &mut crate::backend::Recorder) -> shimmer_b200::Result<shimmer_b200::TextureId> {\n"
 REC_M = "    fn record(&self, r: &mut crate::backend::Recorder) -> shimmer_b200::Result<shimmer_b200::MaterialId> {\n"
@@ -156,6 +155,10 @@ EDITS = {
 
 
 def main():
+    if not 2 <= len(sys.argv) <= 3:
+        sys.exit(__doc__)
+    REF = Path(sys.argv[1])
+    OUT = Path(sys.argv[2]) if len(sys.argv) > 2 else HERE / "shimmer-b200.patch"
     tmp = Path(tempfile.mkdtemp(prefix="shimmer_patch_"))
     for side in ("a", "b"):
         (tmp / side).mkdir()
@@ -176,9 +179,9 @@ def main():
         if ln.startswith(("--- a/", "+++ b/", "--- b/", "+++ a/")):
             ln = ln.split("\t")[0].rstrip("\n") + "\n"
         lines.append(ln)
-    (HERE / "shimmer-b200.patch").write_text("".join(lines))
+    OUT.write_text("".join(lines))
     shutil.rmtree(tmp)
-    print(f"wrote {HERE / 'shimmer-b200.patch'}: {sum(1 for l in lines if l.startswith('+') and not l.startswith('+++'))} added lines, "
+    print(f"wrote {OUT}: {sum(1 for l in lines if l.startswith('+') and not l.startswith('+++'))} added lines, "
           f"{sum(1 for l in lines if l.startswith('-') and not l.startswith('---'))} removed")
 
 

@@ -1,5 +1,6 @@
 """The Rust -sys crate (rust/shimmer-b200-sys, sources only: no rustc in this image) must declare exactly what
 include/shimmer_b200.h declares: same symbols, same arity, same struct fields in the same order, same constants."""
+import os
 import re
 from pathlib import Path
 
@@ -74,22 +75,25 @@ def test_library_exports_what_the_rust_crate_links_against():
         assert hasattr(lib, name), name
 
 
+PATCH = ROOT / "rust" / "shimmer-patch" / "shimmer-b200.patch"
+# the reference crate's files the patch changes, as far as the patch and make_patch.py record them
+# (tests/golden/make_reference_excerpt.py); SHIMMER_REFERENCE_DIR may name a full checkout instead
+REFERENCE = Path(os.environ.get("SHIMMER_REFERENCE_DIR") or ROOT / "tests" / "golden" / "reference_excerpt")
+
+
 def test_reference_patch_applies_cleanly(tmp_path):
     """rust/shimmer-patch/shimmer-b200.patch (the `record` method of every implementor, Bvh upload, Camera POD, the new
-    body of Renderer::render, src/backend.rs) applies to a pristine copy of the reference crate and is what
-    make_patch.py generates from it.  No Rust toolchain exists in this image: applying is all that can be checked."""
+    body of Renderer::render, src/backend.rs) applies to the reference crate without fuzz and is what make_patch.py
+    generates from it.  The Rust code is applied, not compiled."""
     import shutil
     import subprocess
-    import pytest
-    ref = Path("/root/reference")
-    if not (ref / "src" / "renderer.rs").exists() or shutil.which("patch") is None:
-        pytest.skip("needs the reference checkout and patch(1)")
-    patch = ROOT / "rust" / "shimmer-patch" / "shimmer-b200.patch"
+    import sys
+    ref = REFERENCE.resolve()
     work = tmp_path / "shimmer"
     work.mkdir()
     shutil.copy(ref / "Cargo.toml", work / "Cargo.toml")
     shutil.copytree(ref / "src", work / "src")
-    out = subprocess.run(["patch", "-p1", "--no-backup-if-mismatch", "-i", str(patch)], cwd=work, capture_output=True, text=True)
+    out = subprocess.run(["patch", "-p1", "--no-backup-if-mismatch", "-i", str(PATCH)], cwd=work, capture_output=True, text=True)
     assert out.returncode == 0 and "FAILED" not in out.stdout and "fuzz" not in out.stdout, out.stdout + out.stderr
     assert (work / "src" / "backend.rs").read_text() == (ROOT / "rust" / "shimmer-patch" / "backend.rs").read_text()
     # every implementor the crate ships overrides `record`: 4 textures, 5 materials, 12 hittables
@@ -97,7 +101,8 @@ def test_reference_patch_applies_cleanly(tmp_path):
     assert n == 4 + 5 + 12, n
     assert "crate::backend::render_on_device(" in (work / "src" / "renderer.rs").read_text()
     # the committed patch is what the generator produces today
-    before = patch.read_text()
-    gen = subprocess.run(["python", str(ROOT / "rust" / "shimmer-patch" / "make_patch.py"), str(ref)], capture_output=True, text=True)
+    regen = tmp_path / "regenerated.patch"
+    gen = subprocess.run([sys.executable, str(ROOT / "rust" / "shimmer-patch" / "make_patch.py"), str(ref), str(regen)],
+                         capture_output=True, text=True)
     assert gen.returncode == 0, gen.stderr
-    assert patch.read_text() == before
+    assert regen.read_bytes() == PATCH.read_bytes()
