@@ -183,6 +183,29 @@ int shim_trace_closest(shim_scene* s, const float* rays, int64_t n, float t_min,
 int shim_trace_closest_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
                               int32_t* d_prim_id, float* d_t, void* cuda_stream);
 
+/* Hittable::hit on the world (hittable.rs:100-118) with the whole HitRecord (hittable.rs:15-52).  48 bytes.
+ * The same rays, walk and Philox stream as shim_trace_closest: `hittable` and `t` equal its prim_id and t bit for bit.
+ * A miss is hittable = -1, material = -1, t = +inf and every other field 0.  The record is what the reference's
+ * hit() chain returns: sphere / moving-sphere uv are always evaluated (sphere.rs:41-46); a RotateY hit carries the
+ * normal set_face_normal gave it with the rotated ray and the front_face of the inner hit, untouched
+ * (instance.rs:124-141); a Translate hit has the offset added to its point (instance.rs:40-42).  A ConstantMedium hit is
+ * normal (1, 0, 0), u = v = 0, front_face = 1 (hittable.rs:216-231), and its material is the Isotropic that
+ * shim_constant_medium allotted: the next material id after those created so far, taken at that call, so a
+ * medium's phase material is numbered among the shim_material_* ids in call order. */
+typedef struct shim_hit_record {
+    float point[3], normal[3];  /* world space; normal face-forwarded as HitRecord::new / set_face_normal leave it */
+    float t, u, v;
+    int32_t front_face;         /* 1 / 0 */
+    int32_t material;           /* material id; a ConstantMedium hit reports the Isotropic that shim_constant_medium allotted */
+    int32_t hittable;           /* the id shim_trace_closest reports; -1 = miss */
+} shim_hit_record;
+int shim_trace_hit(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                   shim_hit_record* out, uint64_t* counters3 /* optional, as shim_trace_closest */);
+/* same on device buffers of the scene's device (it must be current), launched on `cuda_stream` (0 = default stream);
+ * d_out must be 16-byte aligned (each record is written as three 16-byte stores) */
+int shim_trace_hit_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                          shim_hit_record* d_out, void* cuda_stream);
+
 /* ---- host helpers that mirror reference functions (no device needed) ------------------- */
 /* Tile::tile, renderer.rs:242-296: writes up to cap tiles as (width, height, x0, y0); returns the count */
 int shim_tile_layout(int image_width, int image_height, int tile_width, int tile_height, int32_t* out4, int cap);

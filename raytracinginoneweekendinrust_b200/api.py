@@ -47,6 +47,28 @@ class Scene(capi.SceneHandle):
             raise ShimError(rc, self.lib.shim_last_error().decode())
         return (prim, t, cnt) if counters else (prim, t)
 
+    def trace_hit(self, rays: np.ndarray, t_min=0.001, t_max=float("inf"), seed=0, counters=False):
+        """``Hittable::hit`` on the world for a batch of rays (n x 7: origin, direction, time) with the whole record:
+        a structured array of ``capi.HIT_RECORD_DTYPE`` (``hittable == -1`` on a miss); with ``counters`` also
+        (rays, node visits, primitive tests) as ``trace_closest`` gives them."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 7)
+        n = rays.shape[0]
+        out = np.empty(n, capi.HIT_RECORD_DTYPE)
+        cnt = np.zeros(3, np.uint64)
+        rc = self.lib.shim_trace_hit(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data_as(C.POINTER(capi.HitRecord)),
+                                     cnt.ctypes.data if counters else None)
+        if rc < 0:
+            raise ShimError(rc, self.lib.shim_last_error().decode())
+        return (out, cnt) if counters else out
+
+    def trace_hit_device(self, d_rays_ptr: int, n: int, d_out_ptr: int, t_min=0.001, t_max=float("inf"), seed=0, stream: int = 0):
+        """``trace_hit`` on device buffers (e.g. ``torch.Tensor.data_ptr()``): ``d_rays_ptr`` n x 7 float32, ``d_out_ptr``
+        n records of 48 bytes, 16-byte aligned.  Enqueued on ``stream``; the scene's device must be current."""
+        rc = self.lib.shim_trace_hit_device(self.ptr, C.c_void_p(d_rays_ptr), n, t_min, t_max, seed,
+                                            C.cast(C.c_void_p(d_out_ptr), C.POINTER(capi.HitRecord)), C.c_void_p(stream))
+        if rc < 0:
+            raise ShimError(rc, self.lib.shim_last_error().decode())
+
     # ---- render
     def render(self, camera: Camera, params: RenderParams, out: np.ndarray | None = None):
         """Blocking render into a host framebuffer; returns (H, W, 3) float32 (row 0 = bottom) and Stats.

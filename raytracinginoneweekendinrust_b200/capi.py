@@ -88,6 +88,24 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class HitRecord(C.Structure):
+    """``shim_hit_record``: the reference's ``HitRecord`` (hittable.rs:15-52) plus the id of what was hit (48 bytes)."""
+
+    _fields_ = [
+        ("point", C.c_float * 3), ("normal", C.c_float * 3), ("t", C.c_float), ("u", C.c_float), ("v", C.c_float),
+        ("front_face", C.c_int32), ("material", C.c_int32), ("hittable", C.c_int32),
+    ]
+
+
+# the same record as a numpy structured dtype (same field offsets as HitRecord)
+HIT_RECORD_DTYPE = np.dtype({
+    "names": [n for n, _ in HitRecord._fields_],
+    "formats": [(np.float32, (3,)), (np.float32, (3,)), np.float32, np.float32, np.float32, np.int32, np.int32, np.int32],
+    "offsets": [getattr(HitRecord, n).offset for n, _ in HitRecord._fields_],
+    "itemsize": C.sizeof(HitRecord),
+})
+
+
 _F, _I, _P = C.c_float, C.c_int, C.c_void_p
 # builder vocabulary shared by the product (shim_) and the test oracle (orc_)
 _BUILDER_SIGS = {
@@ -173,6 +191,10 @@ def load_library() -> C.CDLL:
     lib.shim_trace_closest.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P, _P]
     lib.shim_trace_closest_device.restype = _I
     lib.shim_trace_closest_device.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P, _P]
+    lib.shim_trace_hit.restype = _I
+    lib.shim_trace_hit.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, C.POINTER(HitRecord), _P]
+    lib.shim_trace_hit_device.restype = _I
+    lib.shim_trace_hit_device.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, C.POINTER(HitRecord), _P]
     lib.shim_tile_layout.restype = _I
     lib.shim_tile_layout.argtypes = [_I, _I, _I, _I, _P, _I]
     lib.shim_camera_fields.restype = _I

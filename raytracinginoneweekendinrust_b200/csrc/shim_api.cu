@@ -1085,3 +1085,66 @@ SHIM_API int shim_trace_closest(shim_scene* s, const float* rays, int64_t n, flo
     cleanup();
     return SHIM_OK;
 }
+
+static_assert(sizeof(shim_hit_record) == 3 * sizeof(f4), "shim_hit_record is three 16-byte words");
+
+// as trace_grid, for the 128-thread blocks of trace_hit_kernel (the same number of threads at most)
+static int trace_hit_grid(const DeviceScene& ds, int64_t n) {
+    int64_t grid = (n + SHIM_TRACE_HIT_THREADS - 1) / SHIM_TRACE_HIT_THREADS;
+    int64_t cap = (int64_t)ds.sm_count * 8 * (256 / SHIM_TRACE_HIT_THREADS);
+    return (int)(grid > cap ? cap : grid);
+}
+
+SHIM_API int shim_trace_hit_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                                   shim_hit_record* d_out, void* cuda_stream) {
+    NEED(s);
+    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_hit: scene not committed");
+    if (n < 0 || (n > 0 && (!d_rays || !d_out))) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: bad arguments");
+    if (((uintptr_t)d_out & 15) != 0) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: d_out is not 16-byte aligned");
+    if (n == 0) return SHIM_OK;
+    int cur_dev = -1;
+    CU(cudaGetDevice(&cur_dev));
+    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, "shim_trace_hit: the scene lives on another CUDA device");
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, cur_dev, &ds);
+    if (rc < 0) return rc;
+    trace_hit_kernel<<<trace_hit_grid(*ds, n), SHIM_TRACE_HIT_THREADS, 0, (cudaStream_t)cuda_stream>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, (f4*)d_out, nullptr);
+    CU(cudaGetLastError());
+    return SHIM_OK;
+}
+
+SHIM_API int shim_trace_hit(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed, shim_hit_record* out,
+                            uint64_t* counters) {
+    NEED(s);
+    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_hit: scene not committed");
+    if (n < 0 || (n > 0 && (!rays || !out))) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: bad arguments");
+    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
+    DeviceGuard guard;
+    CU(guard.enter(s->dev->primary));
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, s->dev->primary, &ds);
+    if (rc < 0) return rc;
+    float* d_rays = nullptr; f4* d_out = nullptr; unsigned long long* d_cnt = nullptr;
+    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_out); cudaFree(d_cnt); };
+#define CUX(call)                                                                                                     \
+    do {                                                                                                              \
+        cudaError_t e_ = (call);                                                                                      \
+        if (e_ != cudaSuccess) { cleanup(); return set_err(SHIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
+    } while (0)
+    CUX(cudaMalloc(&d_rays, (size_t)n * 7 * sizeof(float)));
+    CUX(cudaMalloc(&d_out, (size_t)n * sizeof(shim_hit_record)));
+    CUX(cudaMalloc(&d_cnt, 3 * sizeof(unsigned long long)));
+    CUX(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
+    CUX(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
+    trace_hit_kernel<<<trace_hit_grid(*ds, n), SHIM_TRACE_HIT_THREADS>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_out, counters ? d_cnt : nullptr);
+    CUX(cudaGetLastError());
+    CUX(cudaMemcpy(out, d_out, (size_t)n * sizeof(shim_hit_record), cudaMemcpyDeviceToHost));
+    if (counters) {
+        unsigned long long h[3];
+        CUX(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
+        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
+    }
+    cleanup();
+    return SHIM_OK;
+#undef CUX
+}

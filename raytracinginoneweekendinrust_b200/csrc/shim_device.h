@@ -870,6 +870,23 @@ SHIM_HD void reconstruct_hit(const SceneView& sv, const Ray& ray, const Hit& h, 
     if (ob.flags & OBJ_TRANSLATE) rec.point = rec.point + mk3(ob.dx, ob.dy, ob.dz);  // instance.rs:40-42
 }
 
+// shim_hit_record (include/shimmer_b200.h) of a closest_hit result as three 16-byte words: {point, normal.x},
+// {normal.yz, t, u}, {v, front_face, material, hittable}.  uv is always evaluated, as the reference's hit() does;
+// material and hittable are the ids hit_material / hit_handle give.  A miss: t = +inf, ids -1, the rest 0.
+SHIM_HD void hit_record_words(const SceneView& sv, const Ray& ray, const Hit& h, f4& w0, f4& w1, f4& w2) {
+    if (h.obj < 0) {
+        w0 = f4{0.0f, 0.0f, 0.0f, 0.0f};
+        w1 = f4{0.0f, 0.0f, SHIM_INF, 0.0f};
+        w2 = f4{0.0f, i2f(0), i2f(-1), i2f(-1)};
+        return;
+    }
+    HitRec rec;
+    reconstruct_hit(sv, ray, h, true, rec);
+    w0 = f4{rec.point.x, rec.point.y, rec.point.z, rec.normal.x};
+    w1 = f4{rec.normal.y, rec.normal.z, rec.t, rec.u};
+    w2 = f4{rec.v, i2f(rec.front_face ? 1 : 0), i2f(hit_material(sv, h)), i2f(hit_handle(sv, h))};
+}
+
 // ---------------------------------------------------------------------------- textures
 // Perlin / Turbulence standing in for the `noise` crate (see DESIGN.md); f64 like the crate.
 SHIM_HD double perlin_fade(double t) { return t * t * t * (t * (t * 6.0 - 15.0) + 10.0); }

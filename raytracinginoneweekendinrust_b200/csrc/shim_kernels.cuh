@@ -1098,4 +1098,34 @@ __global__ void __launch_bounds__(256) trace_closest_kernel(SceneView sv, const 
     }
 }
 
+// Hittable::hit with the whole record for a batch of rays: the walk and the Philox keying of trace_closest_kernel,
+// then the HitRecord rebuilt in registers and written as three 16-byte stores per ray (out: 3 f4 per ray).
+// 128-thread blocks, three per SM: 158 registers and no spills (at the 128 registers of two 256-thread blocks the
+// walk plus the record spill 88 bytes).
+#define SHIM_TRACE_HIT_THREADS 128
+__global__ void __launch_bounds__(SHIM_TRACE_HIT_THREADS, 3) trace_hit_kernel(SceneView sv, const float* rays, long long n, float t_min, float t_max,
+                                                        uint64_t seed, f4* out, unsigned long long* counters) {
+    uint32_t nodes = 0, prims = 0;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const float* q = rays + i * 7;
+        Ray r; r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
+        Rng rng;
+        rng_init(rng, (uint32_t)i, 0, seed);
+        rng_key(rng, 0, STAGE_INTERSECT);
+        TraceCounters tc; tc.nodes = 0; tc.prims = 0; tc.hrpp_tp = 0; tc.hrpp_fp = 0; tc.hrpp_none = 0;
+        Hit h = counters ? closest_hit<true>(sv, r, t_min, t_max, rng, &tc)
+                         : (sv.qnodes ? closest_hit<false, false, true, true>(sv, r, t_min, t_max, rng, &tc) : closest_hit<false>(sv, r, t_min, t_max, rng, &tc));
+        nodes += tc.nodes; prims += tc.prims;
+        f4 w0, w1, w2;
+        hit_record_words(sv, r, h, w0, w1, w2);
+        out[3 * i] = w0;
+        out[3 * i + 1] = w1;
+        out[3 * i + 2] = w2;
+    }
+    if (counters) {
+        atomicAdd(counters + 1, (unsigned long long)nodes);
+        atomicAdd(counters + 2, (unsigned long long)prims);
+    }
+}
+
 }  // namespace shim

@@ -88,6 +88,21 @@ pub struct shim_stats {
     pub wall_ms: f64,
 }
 
+/// `Hittable::hit`'s `HitRecord` (hittable.rs:15-52) plus the id of what was hit; 48 bytes (`shim_trace_hit`).
+/// `hittable == -1`: a miss (`material == -1`, `t == +inf`, everything else 0).
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct shim_hit_record {
+    pub point: [f32; 3],
+    pub normal: [f32; 3],
+    pub t: f32,
+    pub u: f32,
+    pub v: f32,
+    pub front_face: i32,
+    pub material: i32,
+    pub hittable: i32,
+}
+
 extern "C" {
     pub fn shim_last_error() -> *const c_char;
     pub fn shim_version() -> c_int;
@@ -159,6 +174,14 @@ extern "C" {
     pub fn shim_trace_closest_device(
         s: *mut shim_scene, d_rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
         d_prim_id: *mut i32, d_t: *mut f32, cuda_stream: *mut c_void,
+    ) -> c_int;
+    pub fn shim_trace_hit(
+        s: *mut shim_scene, rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
+        out: *mut shim_hit_record, counters3: *mut u64,
+    ) -> c_int;
+    pub fn shim_trace_hit_device(
+        s: *mut shim_scene, d_rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
+        d_out: *mut shim_hit_record, cuda_stream: *mut c_void,
     ) -> c_int;
 
     pub fn shim_tile_layout(image_width: c_int, image_height: c_int, tile_width: c_int, tile_height: c_int, out4: *mut i32, cap: c_int) -> c_int;

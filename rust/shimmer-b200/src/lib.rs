@@ -1,7 +1,8 @@
 //! Safe wrapper over the C ABI (`include/shimmer_b200.h`).  One method per reference constructor; ids are plain
 //! newtypes; every call maps `< 0` to `Error` with the library's message.  There is no CPU fallback: without a CUDA
 //! device `commit`/`render` return `Error { code: SHIM_ERR_CUDA, .. }`.
-//! NOTE: written without a Rust toolchain at hand (the build image has none); see rust/README.md.
+//! NOTE: written without a Rust toolchain at hand (the build image has none), so this crate, `trace_hit` included, has
+//! never been compiled; see rust/README.md.
 use std::ffi::{CStr, CString};
 use std::ops::{Deref, DerefMut};
 use std::os::raw::c_int;
@@ -45,6 +46,20 @@ pub struct MaterialId(pub i32);
 /// Also the primitive id `trace_closest` reports.
 #[derive(Clone, Copy, Debug, PartialEq, Eq, Hash)]
 pub struct HittableId(pub i32);
+
+/// `HitRecord` (hittable.rs:15-52) as `Scene::trace_hit` returns it, with the id of the hittable that answered (the id
+/// `trace_closest` reports; a ConstantMedium hit: the medium's id and the Isotropic `constant_medium` allotted).
+#[derive(Clone, Copy, Debug, PartialEq)]
+pub struct HitRecord {
+    pub point: [f32; 3],
+    pub normal: [f32; 3],
+    pub t: f32,
+    pub u: f32,
+    pub v: f32,
+    pub front_face: bool,
+    pub material: MaterialId,
+    pub hittable: HittableId,
+}
 
 /// A scene being recorded, then committed to the current CUDA device.  Not `Sync`: one caller per handle.
 pub struct Scene {
@@ -195,6 +210,33 @@ impl Scene {
             sys::shim_trace_closest(self.raw, rays.as_ptr(), n as i64, t_min, t_max, seed, prim.as_mut_ptr(), t.as_mut_ptr(), std::ptr::null_mut())
         })?;
         Ok((prim, t))
+    }
+    /// `Hittable::hit` on the world for each of `rays` (7 floats each) with the whole record; `None` = no hit, as
+    /// `Option<HitRecord>` in the reference.  Same walk and Philox stream as `trace_closest`.
+    pub fn trace_hit(&mut self, rays: &[f32], t_min: f32, t_max: f32, seed: u64) -> Result<Vec<Option<HitRecord>>> {
+        if rays.len() % 7 != 0 {
+            return Err(Error { code: sys::SHIM_ERR_INVALID, message: "trace_hit: 7 floats per ray".into() });
+        }
+        let n = rays.len() / 7;
+        let mut raw = vec![sys::shim_hit_record::default(); n];
+        check(unsafe {
+            sys::shim_trace_hit(self.raw, rays.as_ptr(), n as i64, t_min, t_max, seed, raw.as_mut_ptr(), std::ptr::null_mut())
+        })?;
+        Ok(raw
+            .iter()
+            .map(|r| {
+                (r.hittable >= 0).then(|| HitRecord {
+                    point: r.point,
+                    normal: r.normal,
+                    t: r.t,
+                    u: r.u,
+                    v: r.v,
+                    front_face: r.front_face != 0,
+                    material: MaterialId(r.material),
+                    hittable: HittableId(r.hittable),
+                })
+            })
+            .collect())
     }
 }
 impl Drop for Scene {
