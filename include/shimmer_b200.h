@@ -206,6 +206,20 @@ int shim_trace_hit(shim_scene* s, const float* rays, int64_t n, float t_min, flo
 int shim_trace_hit_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
                           shim_hit_record* d_out, void* cuda_stream);
 
+/* Occlusion (any hit): is anything hit on the ray with t in [t_min, t_max]?  occluded[i] = 1 / 0, one byte per ray.
+ * The walk stops at the first hit it accepts instead of searching for the closest one, on the same rays, node layouts
+ * and Philox stream as shim_trace_closest (a medium draws its free path from the same stream), and
+ *     occluded[i] == (shim_trace_closest(s, rays, n, t_min, t_max, seed, ...).prim_id[i] >= 0)
+ * for every ray, bit for bit; its node visits and primitive tests (counters3) are never more than that query's.
+ * Visibility between two points a and b (shadow rays, ambient occlusion, "can the camera see p"): origin = a,
+ * direction = b - a (not normalised), t in [eps, 1 - eps], e.g. eps = 1e-3; occluded = 0 means a sees b.
+ * Errors as shim_trace_closest; nothing is written on error. */
+int shim_trace_occluded(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                        uint8_t* occluded, uint64_t* counters3 /* optional: rays, node visits, prim tests */);
+/* same on device buffers of the scene's device (it must be current), launched on `cuda_stream` (0 = default stream) */
+int shim_trace_occluded_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                               uint8_t* d_occluded, void* cuda_stream);
+
 /* ---- host helpers that mirror reference functions (no device needed) ------------------- */
 /* Tile::tile, renderer.rs:242-296: writes up to cap tiles as (width, height, x0, y0); returns the count */
 int shim_tile_layout(int image_width, int image_height, int tile_width, int tile_height, int32_t* out4, int cap);

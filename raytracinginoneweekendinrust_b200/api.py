@@ -69,6 +69,30 @@ class Scene(capi.SceneHandle):
         if rc < 0:
             raise ShimError(rc, self.lib.shim_last_error().decode())
 
+    def trace_occluded(self, rays: np.ndarray, t_min=0.001, t_max=float("inf"), seed=0, counters=False):
+        """Is anything hit on each ray (n x 7: origin, direction, time) with t in [t_min, t_max]?  A bool array, True
+        exactly where ``trace_closest`` of the same rays and seed reports a hit; the walk stops at the first hit found.
+        With ``counters`` also (rays, node visits, primitive tests), never more than ``trace_closest``'s.  Visibility
+        between points a and b: origin a, direction b - a, ``t_min=1e-3, t_max=1 - 1e-3``."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 7)
+        n = rays.shape[0]
+        out = np.empty(n, np.uint8)
+        cnt = np.zeros(3, np.uint64)
+        rc = self.lib.shim_trace_occluded(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data,
+                                          cnt.ctypes.data if counters else None)
+        if rc < 0:
+            raise ShimError(rc, self.lib.shim_last_error().decode())
+        occ = out.view(np.bool_)
+        return (occ, cnt) if counters else occ
+
+    def trace_occluded_device(self, d_rays_ptr: int, n: int, d_out_ptr: int, t_min=0.001, t_max=float("inf"), seed=0, stream: int = 0):
+        """``trace_occluded`` on device buffers (e.g. ``torch.Tensor.data_ptr()``): ``d_rays_ptr`` n x 7 float32,
+        ``d_out_ptr`` n bytes (uint8 or bool: 1 = occluded).  Enqueued on ``stream``; the scene's device must be current."""
+        rc = self.lib.shim_trace_occluded_device(self.ptr, C.c_void_p(d_rays_ptr), n, t_min, t_max, seed, C.c_void_p(d_out_ptr),
+                                                 C.c_void_p(stream))
+        if rc < 0:
+            raise ShimError(rc, self.lib.shim_last_error().decode())
+
     # ---- render
     def render(self, camera: Camera, params: RenderParams, out: np.ndarray | None = None):
         """Blocking render into a host framebuffer; returns (H, W, 3) float32 (row 0 = bottom) and Stats.

@@ -195,6 +195,10 @@ def load_library() -> C.CDLL:
     lib.shim_trace_hit.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, C.POINTER(HitRecord), _P]
     lib.shim_trace_hit_device.restype = _I
     lib.shim_trace_hit_device.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, C.POINTER(HitRecord), _P]
+    lib.shim_trace_occluded.restype = _I
+    lib.shim_trace_occluded.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P]
+    lib.shim_trace_occluded_device.restype = _I
+    lib.shim_trace_occluded_device.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P]
     lib.shim_tile_layout.restype = _I
     lib.shim_tile_layout.argtypes = [_I, _I, _I, _I, _P, _I]
     lib.shim_camera_fields.restype = _I

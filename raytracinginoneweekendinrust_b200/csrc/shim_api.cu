@@ -1148,3 +1148,60 @@ SHIM_API int shim_trace_hit(shim_scene* s, const float* rays, int64_t n, float t
     return SHIM_OK;
 #undef CUX
 }
+
+static_assert(SHIM_TRACE_OCCLUDED_THREADS == 256, "trace_grid sizes the grid for 256-thread blocks");
+
+SHIM_API int shim_trace_occluded_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
+                                        uint8_t* d_occluded, void* cuda_stream) {
+    NEED(s);
+    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: scene not committed");
+    if (n < 0 || (n > 0 && (!d_rays || !d_occluded))) return set_err(SHIM_ERR_INVALID, "shim_trace_occluded: bad arguments");
+    if (n == 0) return SHIM_OK;
+    int cur_dev = -1;
+    CU(cudaGetDevice(&cur_dev));
+    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: the scene lives on another CUDA device");
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, cur_dev, &ds);
+    if (rc < 0) return rc;
+    trace_occluded_kernel<<<trace_grid(*ds, n), SHIM_TRACE_OCCLUDED_THREADS, 0, (cudaStream_t)cuda_stream>>>(ds->view, d_rays, (long long)n, t_min,
+                                                                                                         t_max, seed, d_occluded, nullptr);
+    CU(cudaGetLastError());
+    return SHIM_OK;
+}
+
+SHIM_API int shim_trace_occluded(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed, uint8_t* occluded,
+                                 uint64_t* counters) {
+    NEED(s);
+    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: scene not committed");
+    if (n < 0 || (n > 0 && (!rays || !occluded))) return set_err(SHIM_ERR_INVALID, "shim_trace_occluded: bad arguments");
+    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
+    DeviceGuard guard;
+    CU(guard.enter(s->dev->primary));
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, s->dev->primary, &ds);
+    if (rc < 0) return rc;
+    float* d_rays = nullptr; uint8_t* d_occ = nullptr; unsigned long long* d_cnt = nullptr;
+    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_occ); cudaFree(d_cnt); };
+#define CUX(call)                                                                                                     \
+    do {                                                                                                              \
+        cudaError_t e_ = (call);                                                                                      \
+        if (e_ != cudaSuccess) { cleanup(); return set_err(SHIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
+    } while (0)
+    CUX(cudaMalloc(&d_rays, (size_t)n * 7 * sizeof(float)));
+    CUX(cudaMalloc(&d_occ, (size_t)n));
+    CUX(cudaMalloc(&d_cnt, 3 * sizeof(unsigned long long)));
+    CUX(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
+    CUX(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
+    trace_occluded_kernel<<<trace_grid(*ds, n), SHIM_TRACE_OCCLUDED_THREADS>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_occ,
+                                                                               counters ? d_cnt : nullptr);
+    CUX(cudaGetLastError());
+    CUX(cudaMemcpy(occluded, d_occ, (size_t)n, cudaMemcpyDeviceToHost));
+    if (counters) {
+        unsigned long long h[3];
+        CUX(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
+        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
+    }
+    cleanup();
+    return SHIM_OK;
+#undef CUX
+}

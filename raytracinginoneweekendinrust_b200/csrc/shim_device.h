@@ -472,7 +472,9 @@ SHIM_HD void slab_pair_q(const uint32_t* w, const RayCtx& c, float t_min, float 
 // Both layouts visit the same nodes in the same order and return the same hit: for a box with min <= max and a finite
 // reciprocal the plane the sign picks IS the smaller of the two products (fma is monotonic), and max/min are
 // associative.
-template <bool COUNT, int ONLY = -1, int SIGNED = 0>
+// ANY: an any-hit query.  It returns at the first primitive the closest-hit walk would accept (best holds it), so it is
+// a prefix of that walk: until a first hit, t_cull == t_max in both and they test the same boxes and primitives.
+template <bool COUNT, int ONLY = -1, int SIGNED = 0, bool ANY = false>
 SHIM_HD bool bvh_closest(const SceneView& sv, int start_node, const RayCtx& c, float t_min, float t_max, BvhBest& best,
                          TraceCounters* cnt) {
     best.t = t_max; best.prim = 0; best.face = 0; best.any = false;
@@ -555,6 +557,7 @@ SHIM_HD bool bvh_closest(const SceneView& sv, int start_node, const RayCtx& c, f
             // f32-rounded best.t); what counts is its f32 t: closer wins, an exact tie goes to the later leaf
             // of the recorded tree (bvh.rs:409-415), anything beyond best.t is not a hit
             if (hit_prim<ONLY>(sv, ref, c, t_min, t_cull, t, face) && !(t > best.t)) {
+                if constexpr (ANY) { best.t = t; best.prim = ref; best.face = face; best.any = true; return true; }
                 bool take = !best.any || t < best.t;
                 if (!take) take = tie_goes_to_candidate<ONLY>(sv, c, t_min, ref, best.prim, t);
                 if (take) { best.t = t; best.prim = ref; best.face = face; best.any = true; t_cull = t + fabsf(t) * 3.8146973e-06f; }
@@ -679,7 +682,8 @@ SHIM_HD bool bvh_closest_predicted(const SceneView& sv, const DevObject& ob, con
 // shape of one top-level object against its object-space ray
 // HASBVH = false: the caller knows the world holds no Bvh object (a flat list like the Cornell scenes)
 // QN: the Bvh object sv.q_object is walked on its quantised nodes (same hit; tests/hostsim pins that)
-template <bool COUNT, bool HRPP, bool HASBVH = true, bool QN = false>
+// ANY: a Bvh object answers with its first accepted primitive (bvh_closest<..., ANY>), not the closest one
+template <bool COUNT, bool HRPP, bool HASBVH = true, bool QN = false, bool ANY = false>
 SHIM_HD bool shape_hit(const SceneView& sv, const DevObject& ob, const RayCtx& c, float t_min, float t_max, float& t, uint32_t& prim,
                        int& face, TraceCounters* cnt) {
     if (!HASBVH || ob.kind == OBJ_PRIM) {
@@ -690,16 +694,19 @@ SHIM_HD bool shape_hit(const SceneView& sv, const DevObject& ob, const RayCtx& c
     }
     BvhBest best;
     bool hit;
-    if (QN && sv.qnodes && ob.ref == sv.objects[sv.q_object].ref) hit = bvh_closest<COUNT, -1, 2>(sv, 0, c, t_min, t_max, best, cnt);
+    if (QN && sv.qnodes && ob.ref == sv.objects[sv.q_object].ref) hit = bvh_closest<COUNT, -1, 2, ANY>(sv, 0, c, t_min, t_max, best, cnt);
     else hit = (HRPP && (ob.flags & OBJ_PREDICTOR)) ? bvh_closest_predicted<COUNT>(sv, ob, c, t_min, t_max, best, cnt)
-                                                    : bvh_closest<COUNT>(sv, ob.ref, c, t_min, t_max, best, cnt);
+                                                    : bvh_closest<COUNT, -1, 0, ANY>(sv, ob.ref, c, t_min, t_max, best, cnt);
     if (hit) { t = best.t; prim = best.prim; face = best.face; return true; }
     return false;
 }
 
 // HittableList::hit over the flattened world (hittable.rs:100-118), with ConstantMedium::hit
 // (hittable.rs:177-233) for medium objects.  `rng` must be keyed to STAGE_INTERSECT.
-template <bool COUNT, bool HRPP = false, bool HASBVH = true, bool QN = false>
+// ANY: the occlusion query - returns at the first object that has a hit (for a medium: once its free path is accepted).
+// Until that object `closest` is t_max, so it makes the closest-hit query's tests and Philox draws, a prefix of them;
+// h.obj >= 0 exactly when the closest-hit query's does.  h is then that first hit, not the closest one.
+template <bool COUNT, bool HRPP = false, bool HASBVH = true, bool QN = false, bool ANY = false>
 SHIM_HD Hit closest_hit(const SceneView& sv, const Ray& ray, float t_min, float t_max, Rng& rng, TraceCounters* cnt) {
     Hit h; h.t = t_max; h.obj = -1; h.prim = 0; h.face = 0;
     float closest = t_max;
@@ -719,7 +726,10 @@ SHIM_HD Hit closest_hit(const SceneView& sv, const Ray& ray, float t_min, float 
 #pragma unroll 1
 #endif
         for (int pass = 0; pass < 2; ++pass) {
-            found = shape_hit<COUNT, HRPP, HASBVH, QN>(sv, ob, c, lo, hi, t, prim, face, cnt);
+            // a medium's boundary stays a closest-hit query: the free path needs its entry and exit t
+            if constexpr (ANY) found = medium ? shape_hit<COUNT, HRPP, HASBVH, QN>(sv, ob, c, lo, hi, t, prim, face, cnt)
+                                              : shape_hit<COUNT, HRPP, HASBVH, QN, true>(sv, ob, c, lo, hi, t, prim, face, cnt);
+            else found = shape_hit<COUNT, HRPP, HASBVH, QN>(sv, ob, c, lo, hi, t, prim, face, cnt);
             if (!found || !medium || pass == 1) break;
             t1 = t; lo = t1 + 0.0001f;
         }
@@ -741,6 +751,7 @@ SHIM_HD Hit closest_hit(const SceneView& sv, const Ray& ray, float t_min, float 
             closest = t;
             h.t = t; h.obj = oi; h.prim = prim; h.face = face;
         }
+        if constexpr (ANY) break;
     }
     return h;
 }

@@ -1128,4 +1128,32 @@ __global__ void __launch_bounds__(SHIM_TRACE_HIT_THREADS, 3) trace_hit_kernel(Sc
     }
 }
 
+// Occlusion (any hit) for a batch of rays: the rays, node layouts and Philox keying of trace_closest_kernel, the walk
+// ending at the first accepted hit (closest_hit<..., ANY = true>).  occluded[i] = 1 exactly where trace_closest_kernel
+// reports prim_id >= 0.  256-thread blocks, two per SM: 128 registers and no spills (with __launch_bounds__(256) alone
+// ptxas also settles on 128 registers but spills 16 bytes, as trace_closest_kernel does).
+#define SHIM_TRACE_OCCLUDED_THREADS 256
+__global__ void __launch_bounds__(SHIM_TRACE_OCCLUDED_THREADS, 2) trace_occluded_kernel(SceneView sv, const float* rays, long long n, float t_min,
+                                                                                     float t_max, uint64_t seed, uint8_t* occluded,
+                                                                                     unsigned long long* counters) {
+    uint32_t nodes = 0, prims = 0;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const float* q = rays + i * 7;
+        Ray r; r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
+        Rng rng;
+        rng_init(rng, (uint32_t)i, 0, seed);
+        rng_key(rng, 0, STAGE_INTERSECT);
+        TraceCounters tc; tc.nodes = 0; tc.prims = 0; tc.hrpp_tp = 0; tc.hrpp_fp = 0; tc.hrpp_none = 0;
+        Hit h = counters ? closest_hit<true, false, true, false, true>(sv, r, t_min, t_max, rng, &tc)
+                         : (sv.qnodes ? closest_hit<false, false, true, true, true>(sv, r, t_min, t_max, rng, &tc)
+                                      : closest_hit<false, false, true, false, true>(sv, r, t_min, t_max, rng, &tc));
+        nodes += tc.nodes; prims += tc.prims;
+        occluded[i] = h.obj >= 0 ? 1 : 0;
+    }
+    if (counters) {
+        atomicAdd(counters + 1, (unsigned long long)nodes);
+        atomicAdd(counters + 2, (unsigned long long)prims);
+    }
+}
+
 }  // namespace shim

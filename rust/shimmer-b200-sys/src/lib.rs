@@ -183,6 +183,14 @@ extern "C" {
         s: *mut shim_scene, d_rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
         d_out: *mut shim_hit_record, cuda_stream: *mut c_void,
     ) -> c_int;
+    pub fn shim_trace_occluded(
+        s: *mut shim_scene, rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
+        occluded: *mut u8, counters3: *mut u64,
+    ) -> c_int;
+    pub fn shim_trace_occluded_device(
+        s: *mut shim_scene, d_rays: *const f32, n: i64, t_min: f32, t_max: f32, seed: u64,
+        d_occluded: *mut u8, cuda_stream: *mut c_void,
+    ) -> c_int;
 
     pub fn shim_tile_layout(image_width: c_int, image_height: c_int, tile_width: c_int, tile_height: c_int, out4: *mut i32, cap: c_int) -> c_int;
     pub fn shim_camera_fields(cam: *const shim_camera, out21: *mut f32) -> c_int;

@@ -1,8 +1,8 @@
 //! Safe wrapper over the C ABI (`include/shimmer_b200.h`).  One method per reference constructor; ids are plain
 //! newtypes; every call maps `< 0` to `Error` with the library's message.  There is no CPU fallback: without a CUDA
 //! device `commit`/`render` return `Error { code: SHIM_ERR_CUDA, .. }`.
-//! NOTE: written without a Rust toolchain at hand (the build image has none), so this crate, `trace_hit` included, has
-//! never been compiled; see rust/README.md.
+//! NOTE: written without a Rust toolchain at hand (the build image has none), so this crate, `trace_hit` and
+//! `trace_occluded` included, has never been compiled; see rust/README.md.
 use std::ffi::{CStr, CString};
 use std::ops::{Deref, DerefMut};
 use std::os::raw::c_int;
@@ -237,6 +237,20 @@ impl Scene {
                 })
             })
             .collect())
+    }
+    /// Occlusion (any hit): is anything hit on each of `rays` (7 floats each) with t in [t_min, t_max]?  `true` exactly
+    /// where `trace_closest` of the same rays and seed reports a hit; the walk stops at the first hit it finds.
+    /// Visibility between points a and b: origin a, direction b - a, t in [1e-3, 1 - 1e-3].
+    pub fn trace_occluded(&mut self, rays: &[f32], t_min: f32, t_max: f32, seed: u64) -> Result<Vec<bool>> {
+        if rays.len() % 7 != 0 {
+            return Err(Error { code: sys::SHIM_ERR_INVALID, message: "trace_occluded: 7 floats per ray".into() });
+        }
+        let n = rays.len() / 7;
+        let mut occ = vec![0u8; n];
+        check(unsafe {
+            sys::shim_trace_occluded(self.raw, rays.as_ptr(), n as i64, t_min, t_max, seed, occ.as_mut_ptr(), std::ptr::null_mut())
+        })?;
+        Ok(occ.iter().map(|&o| o != 0).collect())
     }
 }
 impl Drop for Scene {
