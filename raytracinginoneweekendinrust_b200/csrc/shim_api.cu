@@ -547,7 +547,8 @@ static void launch_tail(const Wavefront& w, const WfParams& k, cudaStream_t st) 
         if (k.solo_only == PT_SPHERE) wf_tail<false, true, PT_SPHERE><<<w.grid_tail, 128, 0, st>>>(); else wf_tail<false, true, -1><<<w.grid_tail, 128, 0, st>>>();
         return;
     }
-    if (k.use_hrpp) wf_tail<true><<<w.grid_tail, 128, 0, st>>>(); else wf_tail<false><<<w.grid_tail, 128, 0, st>>>();
+    if (k.count_nodes) wf_tail<false, false, -1, true><<<w.grid_tail, 128, 0, st>>>();   // never with k.solo or k.use_hrpp
+    else if (k.use_hrpp) wf_tail<true><<<w.grid_tail, 128, 0, st>>>(); else wf_tail<false><<<w.grid_tail, 128, 0, st>>>();
 }
 static void launch_trace(const Wavefront& w, const WfParams& k, cudaStream_t st) {
     if (k.solo_only == PT_SPHERE) wf_trace_solo<SHIM_SOLO_SPHERE_THREADS, PT_SPHERE><<<w.sm_count, SHIM_SOLO_SPHERE_THREADS, k.smem.total, st>>>();

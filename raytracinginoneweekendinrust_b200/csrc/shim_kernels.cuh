@@ -819,7 +819,9 @@ __device__ __forceinline__ void trace_finish(const WfParams& p) {
 __global__ void wf_trace_first() {   // before the loop: the counters of iteration 0
     if (blockIdx.x == 0 && threadIdx.x == 0) { trace_prepare_iteration(g_p); __threadfence(); }
 }
-template <bool HRPP, bool SOLO = false, int ONLY = -1>
+// COUNT: node visits and primitive tests of the endgame's walks go to C64_NODES / C64_PRIMS like wf_extend's (a counted
+// render: SHIM_RENDER_COUNT_NODES)
+template <bool HRPP, bool SOLO = false, int ONLY = -1, bool COUNT = false>
 __global__ void __launch_bounds__(128) wf_tail() {
     const WfParams& p = g_p;
     const int cur = (int)p.cnt[CNT_CUR];
@@ -843,7 +845,9 @@ __global__ void __launch_bounds__(128) wf_tail() {
             rng_key(rng, (uint32_t)bounce, STAGE_INTERSECT);
             ++traced;
             if (ray_has_nan(r)) break;  // see extend_rays
-            Hit h = SOLO ? closest_hit_solo<false, ONLY>(p.sv, r, 0.001f, SHIM_INF, &tc) : closest_hit<false, HRPP>(p.sv, r, 0.001f, SHIM_INF, rng, &tc);
+            Hit h;
+            if constexpr (COUNT) h = closest_hit<true, false>(p.sv, r, 0.001f, SHIM_INF, rng, &tc);
+            else h = SOLO ? closest_hit_solo<false, ONLY>(p.sv, r, 0.001f, SHIM_INF, &tc) : closest_hit<false, HRPP>(p.sv, r, 0.001f, SHIM_INF, rng, &tc);
             if (h.obj < 0) {
                 float* a = p.accum + 3 * (size_t)pixel;
                 atomicAdd(a + 0, thr.x * p.bg[0]);
@@ -872,6 +876,10 @@ __global__ void __launch_bounds__(128) wf_tail() {
     unsigned long long extra = traced;
     for (int off = 16; off > 0; off >>= 1) extra += __shfl_down_sync(0xffffffffu, extra, off);
     if ((threadIdx.x & 31) == 0 && extra) atomicAdd(cnt64(p.cnt, C64_RAYS), extra);
+    if constexpr (COUNT) {
+        atomicAdd(cnt64(p.cnt, C64_NODES), (unsigned long long)tc.nodes);
+        atomicAdd(cnt64(p.cnt, C64_PRIMS), (unsigned long long)tc.prims);
+    }
     if (HRPP) {
         if (tc.hrpp_tp) atomicAdd(cnt64(p.cnt, C64_HRPP_TP), (unsigned long long)tc.hrpp_tp);
         if (tc.hrpp_fp) atomicAdd(cnt64(p.cnt, C64_HRPP_FP), (unsigned long long)tc.hrpp_fp);
