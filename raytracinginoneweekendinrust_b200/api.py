@@ -41,10 +41,8 @@ class Scene(capi.SceneHandle):
         prim = np.empty(n, np.int32)
         t = np.empty(n, np.float32)
         cnt = np.zeros(3, np.uint64)
-        rc = self.lib.shim_trace_closest(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, prim.ctypes.data, t.ctypes.data,
-                                         cnt.ctypes.data if counters else None)
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("trace_closest", rays.ctypes.data, n, t_min, t_max, seed, prim.ctypes.data, t.ctypes.data,
+                   cnt.ctypes.data if counters else None)
         return (prim, t, cnt) if counters else (prim, t)
 
     def trace_hit(self, rays: np.ndarray, t_min=0.001, t_max=float("inf"), seed=0, counters=False):
@@ -55,19 +53,15 @@ class Scene(capi.SceneHandle):
         n = rays.shape[0]
         out = np.empty(n, capi.HIT_RECORD_DTYPE)
         cnt = np.zeros(3, np.uint64)
-        rc = self.lib.shim_trace_hit(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data_as(C.POINTER(capi.HitRecord)),
-                                     cnt.ctypes.data if counters else None)
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("trace_hit", rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data_as(C.POINTER(capi.HitRecord)),
+                   cnt.ctypes.data if counters else None)
         return (out, cnt) if counters else out
 
     def trace_hit_device(self, d_rays_ptr: int, n: int, d_out_ptr: int, t_min=0.001, t_max=float("inf"), seed=0, stream: int = 0):
         """``trace_hit`` on device buffers (e.g. ``torch.Tensor.data_ptr()``): ``d_rays_ptr`` n x 7 float32, ``d_out_ptr``
         n records of 48 bytes, 16-byte aligned.  Enqueued on ``stream``; the scene's device must be current."""
-        rc = self.lib.shim_trace_hit_device(self.ptr, C.c_void_p(d_rays_ptr), n, t_min, t_max, seed,
-                                            C.cast(C.c_void_p(d_out_ptr), C.POINTER(capi.HitRecord)), C.c_void_p(stream))
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("trace_hit_device", C.c_void_p(d_rays_ptr), n, t_min, t_max, seed,
+                   C.cast(C.c_void_p(d_out_ptr), C.POINTER(capi.HitRecord)), C.c_void_p(stream))
 
     def trace_occluded(self, rays: np.ndarray, t_min=0.001, t_max=float("inf"), seed=0, counters=False):
         """Is anything hit on each ray (n x 7: origin, direction, time) with t in [t_min, t_max]?  A bool array, True
@@ -78,20 +72,16 @@ class Scene(capi.SceneHandle):
         n = rays.shape[0]
         out = np.empty(n, np.uint8)
         cnt = np.zeros(3, np.uint64)
-        rc = self.lib.shim_trace_occluded(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data,
-                                          cnt.ctypes.data if counters else None)
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("trace_occluded", rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data,
+                   cnt.ctypes.data if counters else None)
         occ = out.view(np.bool_)
         return (occ, cnt) if counters else occ
 
     def trace_occluded_device(self, d_rays_ptr: int, n: int, d_out_ptr: int, t_min=0.001, t_max=float("inf"), seed=0, stream: int = 0):
         """``trace_occluded`` on device buffers (e.g. ``torch.Tensor.data_ptr()``): ``d_rays_ptr`` n x 7 float32,
         ``d_out_ptr`` n bytes (uint8 or bool: 1 = occluded).  Enqueued on ``stream``; the scene's device must be current."""
-        rc = self.lib.shim_trace_occluded_device(self.ptr, C.c_void_p(d_rays_ptr), n, t_min, t_max, seed, C.c_void_p(d_out_ptr),
-                                                 C.c_void_p(stream))
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("trace_occluded_device", C.c_void_p(d_rays_ptr), n, t_min, t_max, seed, C.c_void_p(d_out_ptr),
+                   C.c_void_p(stream))
 
     # ---- render
     def render(self, camera: Camera, params: RenderParams, out: np.ndarray | None = None):
@@ -101,9 +91,7 @@ class Scene(capi.SceneHandle):
             out = np.empty((params.height, params.width, 3), np.float32)
         assert out.dtype == np.float32 and out.flags["C_CONTIGUOUS"] and out.shape == (params.height, params.width, 3)
         st = Stats()
-        rc = self.lib.shim_render(self.ptr, C.byref(camera), C.byref(params), out.ctypes.data, C.byref(st))
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("render", C.byref(camera), C.byref(params), out.ctypes.data, C.byref(st))
         return out, st
 
     def render_multi(self, camera: Camera, params: RenderParams, n_devices: int = 0, devices=None, mode: str = "samples",
@@ -118,19 +106,15 @@ class Scene(capi.SceneHandle):
             dev = (C.c_int * len(devices))(*devices)
             n_devices = len(devices)
         st = Stats()
-        rc = self.lib.shim_render_multi(self.ptr, C.byref(camera), C.byref(params), n_devices, dev,
-                                        {"samples": capi.SHARD_SAMPLES, "tiles": capi.SHARD_TILES}[mode], out.ctypes.data, C.byref(st))
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("render_multi", C.byref(camera), C.byref(params), n_devices, dev,
+                   {"samples": capi.SHARD_SAMPLES, "tiles": capi.SHARD_TILES}[mode], out.ctypes.data, C.byref(st))
         return out, st
 
     def render_device(self, camera: Camera, params: RenderParams, d_out_ptr: int, stream: int = 0) -> Stats:
         """Render into a device buffer (e.g. ``torch.Tensor.data_ptr()``) on ``stream``."""
         st = Stats()
-        rc = self.lib.shim_render_device(self.ptr, C.byref(camera), C.byref(params), C.c_void_p(d_out_ptr), C.byref(st),
-                                         C.c_void_p(stream))
-        if rc < 0:
-            raise ShimError(rc, self.lib.shim_last_error().decode())
+        self._call("render_device", C.byref(camera), C.byref(params), C.c_void_p(d_out_ptr), C.byref(st),
+                   C.c_void_p(stream))
         return st
 
 

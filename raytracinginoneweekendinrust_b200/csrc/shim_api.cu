@@ -1027,182 +1027,136 @@ SHIM_API float* shim_host_alloc(size_t floats) {
 SHIM_API void shim_host_free(float* p) { if (p) cudaFreeHost(p); }
 
 // ------------------------------------------------------------------------------------------ gate 1
-static int trace_grid(const DeviceScene& ds, int64_t n) {
-    int grid = (int)((n + 255) / 256);
-    int cap = ds.sm_count * 8;
-    return grid > cap ? cap : grid;
+// Blocks of `threads` for n rays, at most sm_count * 8 blocks' worth of 256 threads; the kernels' grid-stride loops
+// take the rest.
+static int trace_grid(const DeviceScene& ds, int64_t n, int threads) {
+    int64_t grid = (n + threads - 1) / threads;
+    int64_t cap = (int64_t)ds.sm_count * 8 * 256 / threads;
+    return (int)(grid > cap ? cap : grid);
+}
+
+// The checks every batch query makes first, in this order: a scene, committed, n >= 0 and, for n > 0, its arrays.
+static int trace_check(shim_scene* s, const char* fn, int64_t n, bool have_arrays) {
+    NEED(s);
+    if (!s->committed) return set_err(SHIM_ERR_STATE, std::string(fn) + ": scene not committed");
+    if (n < 0 || (n > 0 && !have_arrays)) return set_err(SHIM_ERR_INVALID, std::string(fn) + ": bad arguments");
+    return SHIM_OK;
+}
+
+// The device variants: the caller's arrays and stream on the scene's device, which must be current; no counters.
+// launch(ds) enqueues the kernel.
+template <class Launch>
+static int trace_device(shim_scene* s, const char* fn, int64_t n, Launch launch) {
+    if (n == 0) return SHIM_OK;
+    int cur_dev = -1;
+    CU(cudaGetDevice(&cur_dev));
+    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, std::string(fn) + ": the scene lives on another CUDA device");
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, cur_dev, &ds);
+    if (rc < 0) return rc;
+    launch(*ds);
+    CU(cudaGetLastError());
+    return SHIM_OK;
+}
+
+// The host variants: the rays staged on the scene's device in one allocation with the outputs and the counters, the
+// kernel run on the legacy default stream, then each output array and the counters copied back.
+// launch(ds, d_rays, d_out, d_cnt) enqueues the kernel; d_out[k] holds n * out[k].bytes bytes, 16-byte aligned.
+struct HostOut { void* p; size_t bytes; };   // one output array and its bytes per ray
+template <int K, class Launch>
+static int trace_host(shim_scene* s, const float* rays, int64_t n, const HostOut (&out)[K], uint64_t* counters, Launch launch) {
+    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
+    DeviceGuard guard;
+    CU(guard.enter(s->dev->primary));
+    DeviceScene* ds = nullptr;
+    int rc = scene_on_device(s, s->dev->primary, &ds);
+    if (rc < 0) return rc;
+    // the counters, each output array, the rays
+    size_t off[K + 1], total = 4 * sizeof(unsigned long long);
+    for (int k = 0; k < K; ++k) { off[k] = total; total += ((size_t)n * out[k].bytes + 15) & ~(size_t)15; }
+    off[K] = total; total += (size_t)n * 7 * sizeof(float);
+    char* base = nullptr;
+    CU(cudaMalloc(&base, total));
+    std::unique_ptr<char, cudaError_t (*)(void*)> staging(base, cudaFree);
+    unsigned long long* d_cnt = (unsigned long long*)base;
+    float* d_rays = (float*)(base + off[K]);
+    void* d_out[K];
+    for (int k = 0; k < K; ++k) d_out[k] = base + off[k];
+    CU(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
+    CU(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
+    launch(*ds, d_rays, d_out, counters ? d_cnt : nullptr);
+    CU(cudaGetLastError());
+    for (int k = 0; k < K; ++k) CU(cudaMemcpy(out[k].p, d_out[k], (size_t)n * out[k].bytes, cudaMemcpyDeviceToHost));
+    if (counters) {
+        unsigned long long h[3];
+        CU(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
+        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
+    }
+    return SHIM_OK;
 }
 
 SHIM_API int shim_trace_closest_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
                                        int32_t* d_prim, float* d_t, void* cuda_stream) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_closest: scene not committed");
-    if (n < 0 || (n > 0 && (!d_rays || !d_prim || !d_t))) return set_err(SHIM_ERR_INVALID, "shim_trace_closest: bad arguments");
-    if (n == 0) return SHIM_OK;
-    int cur_dev = -1;
-    CU(cudaGetDevice(&cur_dev));
-    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, "shim_trace_closest: the scene lives on another CUDA device");
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, cur_dev, &ds);
+    int rc = trace_check(s, "shim_trace_closest", n, d_rays && d_prim && d_t);
     if (rc < 0) return rc;
-    trace_closest_kernel<<<trace_grid(*ds, n), 256, 0, (cudaStream_t)cuda_stream>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_prim, d_t, nullptr);
-    CU(cudaGetLastError());
-    return SHIM_OK;
+    return trace_device(s, "shim_trace_closest", n, [&](const DeviceScene& ds) {
+        trace_closest_kernel<<<trace_grid(ds, n, 256), 256, 0, (cudaStream_t)cuda_stream>>>(ds.view, d_rays, (long long)n, t_min, t_max, seed,
+                                                                                             d_prim, d_t, nullptr);
+    });
 }
 
 SHIM_API int shim_trace_closest(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed, int32_t* prim,
                                 float* t, uint64_t* counters) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_closest: scene not committed");
-    if (n < 0 || (n > 0 && (!rays || !prim || !t))) return set_err(SHIM_ERR_INVALID, "shim_trace_closest: bad arguments");
-    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
-    DeviceGuard guard;
-    CU(guard.enter(s->dev->primary));
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, s->dev->primary, &ds);
+    int rc = trace_check(s, "shim_trace_closest", n, rays && prim && t);
     if (rc < 0) return rc;
-    float* d_rays = nullptr; int32_t* d_prim = nullptr; float* d_t = nullptr; unsigned long long* d_cnt = nullptr;
-    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_prim); cudaFree(d_t); cudaFree(d_cnt); };
-#define CUX(call)                                                                                                     \
-    do {                                                                                                              \
-        cudaError_t e_ = (call);                                                                                      \
-        if (e_ != cudaSuccess) { cleanup(); return set_err(SHIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
-    } while (0)
-    CUX(cudaMalloc(&d_rays, (size_t)n * 7 * sizeof(float)));
-    CUX(cudaMalloc(&d_prim, (size_t)n * sizeof(int32_t)));
-    CUX(cudaMalloc(&d_t, (size_t)n * sizeof(float)));
-    CUX(cudaMalloc(&d_cnt, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
-    trace_closest_kernel<<<trace_grid(*ds, n), 256>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_prim, d_t, counters ? d_cnt : nullptr);
-    CUX(cudaGetLastError());
-    CUX(cudaMemcpy(prim, d_prim, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    CUX(cudaMemcpy(t, d_t, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
-    if (counters) {
-        unsigned long long h[3];
-        CUX(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
-        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
-    }
-    cleanup();
-    return SHIM_OK;
+    return trace_host(s, rays, n, {{prim, sizeof *prim}, {t, sizeof *t}}, counters,
+                      [&](const DeviceScene& ds, const float* d_rays, void* const* d_out, unsigned long long* d_cnt) {
+        trace_closest_kernel<<<trace_grid(ds, n, 256), 256>>>(ds.view, d_rays, (long long)n, t_min, t_max, seed, (int32_t*)d_out[0],
+                                                              (float*)d_out[1], d_cnt);
+    });
 }
 
 static_assert(sizeof(shim_hit_record) == 3 * sizeof(f4), "shim_hit_record is three 16-byte words");
 
-// as trace_grid, for the 128-thread blocks of trace_hit_kernel (the same number of threads at most)
-static int trace_hit_grid(const DeviceScene& ds, int64_t n) {
-    int64_t grid = (n + SHIM_TRACE_HIT_THREADS - 1) / SHIM_TRACE_HIT_THREADS;
-    int64_t cap = (int64_t)ds.sm_count * 8 * (256 / SHIM_TRACE_HIT_THREADS);
-    return (int)(grid > cap ? cap : grid);
-}
-
 SHIM_API int shim_trace_hit_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
                                    shim_hit_record* d_out, void* cuda_stream) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_hit: scene not committed");
-    if (n < 0 || (n > 0 && (!d_rays || !d_out))) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: bad arguments");
-    if (((uintptr_t)d_out & 15) != 0) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: d_out is not 16-byte aligned");
-    if (n == 0) return SHIM_OK;
-    int cur_dev = -1;
-    CU(cudaGetDevice(&cur_dev));
-    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, "shim_trace_hit: the scene lives on another CUDA device");
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, cur_dev, &ds);
+    int rc = trace_check(s, "shim_trace_hit", n, d_rays && d_out);
     if (rc < 0) return rc;
-    trace_hit_kernel<<<trace_hit_grid(*ds, n), SHIM_TRACE_HIT_THREADS, 0, (cudaStream_t)cuda_stream>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, (f4*)d_out, nullptr);
-    CU(cudaGetLastError());
-    return SHIM_OK;
+    if (((uintptr_t)d_out & 15) != 0) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: d_out is not 16-byte aligned");
+    return trace_device(s, "shim_trace_hit", n, [&](const DeviceScene& ds) {
+        trace_hit_kernel<<<trace_grid(ds, n, SHIM_TRACE_HIT_THREADS), SHIM_TRACE_HIT_THREADS, 0, (cudaStream_t)cuda_stream>>>(
+            ds.view, d_rays, (long long)n, t_min, t_max, seed, (f4*)d_out, nullptr);
+    });
 }
 
 SHIM_API int shim_trace_hit(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed, shim_hit_record* out,
                             uint64_t* counters) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_hit: scene not committed");
-    if (n < 0 || (n > 0 && (!rays || !out))) return set_err(SHIM_ERR_INVALID, "shim_trace_hit: bad arguments");
-    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
-    DeviceGuard guard;
-    CU(guard.enter(s->dev->primary));
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, s->dev->primary, &ds);
+    int rc = trace_check(s, "shim_trace_hit", n, rays && out);
     if (rc < 0) return rc;
-    float* d_rays = nullptr; f4* d_out = nullptr; unsigned long long* d_cnt = nullptr;
-    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_out); cudaFree(d_cnt); };
-#define CUX(call)                                                                                                     \
-    do {                                                                                                              \
-        cudaError_t e_ = (call);                                                                                      \
-        if (e_ != cudaSuccess) { cleanup(); return set_err(SHIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
-    } while (0)
-    CUX(cudaMalloc(&d_rays, (size_t)n * 7 * sizeof(float)));
-    CUX(cudaMalloc(&d_out, (size_t)n * sizeof(shim_hit_record)));
-    CUX(cudaMalloc(&d_cnt, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
-    trace_hit_kernel<<<trace_hit_grid(*ds, n), SHIM_TRACE_HIT_THREADS>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_out, counters ? d_cnt : nullptr);
-    CUX(cudaGetLastError());
-    CUX(cudaMemcpy(out, d_out, (size_t)n * sizeof(shim_hit_record), cudaMemcpyDeviceToHost));
-    if (counters) {
-        unsigned long long h[3];
-        CUX(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
-        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
-    }
-    cleanup();
-    return SHIM_OK;
-#undef CUX
+    return trace_host(s, rays, n, {{out, sizeof *out}}, counters,
+                      [&](const DeviceScene& ds, const float* d_rays, void* const* d_out, unsigned long long* d_cnt) {
+        trace_hit_kernel<<<trace_grid(ds, n, SHIM_TRACE_HIT_THREADS), SHIM_TRACE_HIT_THREADS>>>(ds.view, d_rays, (long long)n, t_min, t_max,
+                                                                                                 seed, (f4*)d_out[0], d_cnt);
+    });
 }
-
-static_assert(SHIM_TRACE_OCCLUDED_THREADS == 256, "trace_grid sizes the grid for 256-thread blocks");
 
 SHIM_API int shim_trace_occluded_device(shim_scene* s, const float* d_rays, int64_t n, float t_min, float t_max, uint64_t seed,
                                         uint8_t* d_occluded, void* cuda_stream) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: scene not committed");
-    if (n < 0 || (n > 0 && (!d_rays || !d_occluded))) return set_err(SHIM_ERR_INVALID, "shim_trace_occluded: bad arguments");
-    if (n == 0) return SHIM_OK;
-    int cur_dev = -1;
-    CU(cudaGetDevice(&cur_dev));
-    if (cur_dev != s->dev->primary) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: the scene lives on another CUDA device");
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, cur_dev, &ds);
+    int rc = trace_check(s, "shim_trace_occluded", n, d_rays && d_occluded);
     if (rc < 0) return rc;
-    trace_occluded_kernel<<<trace_grid(*ds, n), SHIM_TRACE_OCCLUDED_THREADS, 0, (cudaStream_t)cuda_stream>>>(ds->view, d_rays, (long long)n, t_min,
-                                                                                                         t_max, seed, d_occluded, nullptr);
-    CU(cudaGetLastError());
-    return SHIM_OK;
+    return trace_device(s, "shim_trace_occluded", n, [&](const DeviceScene& ds) {
+        trace_occluded_kernel<<<trace_grid(ds, n, SHIM_TRACE_OCCLUDED_THREADS), SHIM_TRACE_OCCLUDED_THREADS, 0, (cudaStream_t)cuda_stream>>>(
+            ds.view, d_rays, (long long)n, t_min, t_max, seed, d_occluded, nullptr);
+    });
 }
 
 SHIM_API int shim_trace_occluded(shim_scene* s, const float* rays, int64_t n, float t_min, float t_max, uint64_t seed, uint8_t* occluded,
                                  uint64_t* counters) {
-    NEED(s);
-    if (!s->committed) return set_err(SHIM_ERR_STATE, "shim_trace_occluded: scene not committed");
-    if (n < 0 || (n > 0 && (!rays || !occluded))) return set_err(SHIM_ERR_INVALID, "shim_trace_occluded: bad arguments");
-    if (n == 0) { if (counters) counters[0] = counters[1] = counters[2] = 0; return SHIM_OK; }
-    DeviceGuard guard;
-    CU(guard.enter(s->dev->primary));
-    DeviceScene* ds = nullptr;
-    int rc = scene_on_device(s, s->dev->primary, &ds);
+    int rc = trace_check(s, "shim_trace_occluded", n, rays && occluded);
     if (rc < 0) return rc;
-    float* d_rays = nullptr; uint8_t* d_occ = nullptr; unsigned long long* d_cnt = nullptr;
-    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_occ); cudaFree(d_cnt); };
-#define CUX(call)                                                                                                     \
-    do {                                                                                                              \
-        cudaError_t e_ = (call);                                                                                      \
-        if (e_ != cudaSuccess) { cleanup(); return set_err(SHIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
-    } while (0)
-    CUX(cudaMalloc(&d_rays, (size_t)n * 7 * sizeof(float)));
-    CUX(cudaMalloc(&d_occ, (size_t)n));
-    CUX(cudaMalloc(&d_cnt, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemset(d_cnt, 0, 3 * sizeof(unsigned long long)));
-    CUX(cudaMemcpy(d_rays, rays, (size_t)n * 7 * sizeof(float), cudaMemcpyHostToDevice));
-    trace_occluded_kernel<<<trace_grid(*ds, n), SHIM_TRACE_OCCLUDED_THREADS>>>(ds->view, d_rays, (long long)n, t_min, t_max, seed, d_occ,
-                                                                               counters ? d_cnt : nullptr);
-    CUX(cudaGetLastError());
-    CUX(cudaMemcpy(occluded, d_occ, (size_t)n, cudaMemcpyDeviceToHost));
-    if (counters) {
-        unsigned long long h[3];
-        CUX(cudaMemcpy(h, d_cnt, sizeof h, cudaMemcpyDeviceToHost));
-        counters[0] = (uint64_t)n; counters[1] = h[1]; counters[2] = h[2];
-    }
-    cleanup();
-    return SHIM_OK;
-#undef CUX
+    return trace_host(s, rays, n, {{occluded, sizeof *occluded}}, counters,
+                      [&](const DeviceScene& ds, const float* d_rays, void* const* d_out, unsigned long long* d_cnt) {
+        trace_occluded_kernel<<<trace_grid(ds, n, SHIM_TRACE_OCCLUDED_THREADS), SHIM_TRACE_OCCLUDED_THREADS>>>(
+            ds.view, d_rays, (long long)n, t_min, t_max, seed, (uint8_t*)d_out[0], d_cnt);
+    });
 }

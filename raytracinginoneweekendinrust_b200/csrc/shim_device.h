@@ -898,6 +898,41 @@ SHIM_HD void hit_record_words(const SceneView& sv, const Ray& ray, const Hit& h,
     w2 = f4{rec.v, i2f(rec.front_face ? 1 : 0), i2f(hit_material(sv, h)), i2f(hit_handle(sv, h))};
 }
 
+// ---------------------------------------------------------------------------- ray-batch queries
+// Ray i of a batch (7 floats: origin, direction, time) and its Philox stream: pixel i, sample 0, bounce 0 of
+// STAGE_INTERSECT.  The batch kernels (trace_batch in shim_kernels.cuh) and the CPU harness both read rays this way.
+SHIM_HD void batch_ray(const float* rays, long long i, uint64_t seed, Ray& r, Rng& rng) {
+    const float* q = rays + i * 7;
+    r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
+    rng_init(rng, (uint32_t)i, 0, seed);
+    rng_key(rng, 0, STAGE_INTERSECT);
+}
+
+// What each query stores for ray i.  shim_trace_closest: the hittable id and t (+inf on a miss).
+struct StoreClosest {
+    int* prim_id; float* t_out;
+    SHIM_HD void operator()(const SceneView& sv, long long i, const Ray&, const Hit& h) const {
+        prim_id[i] = hit_handle(sv, h);
+        t_out[i] = h.obj < 0 ? SHIM_INF : h.t;
+    }
+};
+// shim_trace_hit: the record as three 16-byte stores (out: 3 f4 per ray).
+struct StoreRecord {
+    f4* out;
+    SHIM_HD void operator()(const SceneView& sv, long long i, const Ray& r, const Hit& h) const {
+        f4 w0, w1, w2;
+        hit_record_words(sv, r, h, w0, w1, w2);
+        out[3 * i] = w0;
+        out[3 * i + 1] = w1;
+        out[3 * i + 2] = w2;
+    }
+};
+// shim_trace_occluded: 1 where the walk accepted a hit.
+struct StoreOccluded {
+    uint8_t* occluded;
+    SHIM_HD void operator()(const SceneView&, long long i, const Ray&, const Hit& h) const { occluded[i] = h.obj >= 0 ? 1 : 0; }
+};
+
 // ---------------------------------------------------------------------------- textures
 // Perlin / Turbulence standing in for the `noise` crate (see DESIGN.md); f64 like the crate.
 SHIM_HD double perlin_fade(double t) { return t * t * t * (t * (t * 6.0 - 15.0) + 10.0); }

@@ -1082,23 +1082,22 @@ __global__ void wf_finalize(const float* accum, float* out, size_t n, float spp,
         out[i] = raw ? accum[i] : accum[i] / spp;
 }
 
-// gate 1: closest hit for a batch of rays
-__global__ void __launch_bounds__(256) trace_closest_kernel(SceneView sv, const float* rays, long long n, float t_min, float t_max,
-                                                            uint64_t seed, int* prim_id, float* t_out, unsigned long long* counters) {
+// gate 1: the grid-stride loop of the three ray-batch queries.  ANY: the occlusion walk, which ends at the first
+// accepted hit (closest_hit<..., ANY = true>).  `store` (StoreClosest / StoreRecord / StoreOccluded) writes ray i's answer.
+template <bool ANY, class Store>
+__device__ __forceinline__ void trace_batch(const SceneView& sv, const float* rays, long long n, float t_min, float t_max, uint64_t seed,
+                                            unsigned long long* counters, Store store) {
     uint32_t nodes = 0, prims = 0;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const float* q = rays + i * 7;
-        Ray r; r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
-        Rng rng;
-        rng_init(rng, (uint32_t)i, 0, seed);
-        rng_key(rng, 0, STAGE_INTERSECT);
+        Ray r; Rng rng;
+        batch_ray(rays, i, seed, r, rng);
         TraceCounters tc; tc.nodes = 0; tc.prims = 0; tc.hrpp_tp = 0; tc.hrpp_fp = 0; tc.hrpp_none = 0;
         // a scene with quantised nodes is queried on them (what its renders walk), unless node visits are being counted
-        Hit h = counters ? closest_hit<true>(sv, r, t_min, t_max, rng, &tc)
-                         : (sv.qnodes ? closest_hit<false, false, true, true>(sv, r, t_min, t_max, rng, &tc) : closest_hit<false>(sv, r, t_min, t_max, rng, &tc));
+        Hit h = counters ? closest_hit<true, false, true, false, ANY>(sv, r, t_min, t_max, rng, &tc)
+                         : (sv.qnodes ? closest_hit<false, false, true, true, ANY>(sv, r, t_min, t_max, rng, &tc)
+                                      : closest_hit<false, false, true, false, ANY>(sv, r, t_min, t_max, rng, &tc));
         nodes += tc.nodes; prims += tc.prims;
-        prim_id[i] = hit_handle(sv, h);
-        t_out[i] = h.obj < 0 ? SHIM_INF : h.t;
+        store(sv, i, r, h);
     }
     if (counters) {
         atomicAdd(counters + 1, (unsigned long long)nodes);
@@ -1106,62 +1105,29 @@ __global__ void __launch_bounds__(256) trace_closest_kernel(SceneView sv, const 
     }
 }
 
-// Hittable::hit with the whole record for a batch of rays: the walk and the Philox keying of trace_closest_kernel,
-// then the HitRecord rebuilt in registers and written as three 16-byte stores per ray (out: 3 f4 per ray).
-// 128-thread blocks, three per SM: 158 registers and no spills (at the 128 registers of two 256-thread blocks the
-// walk plus the record spill 88 bytes).
+// closest hit for a batch of rays
+__global__ void __launch_bounds__(256) trace_closest_kernel(SceneView sv, const float* rays, long long n, float t_min, float t_max,
+                                                            uint64_t seed, int* prim_id, float* t_out, unsigned long long* counters) {
+    trace_batch<false>(sv, rays, n, t_min, t_max, seed, counters, StoreClosest{prim_id, t_out});
+}
+
+// Hittable::hit with the whole record for a batch of rays: the walk of trace_closest_kernel, then the HitRecord rebuilt
+// in registers.  128-thread blocks, three per SM: 158 registers and no spills (at the 128 registers of two 256-thread
+// blocks the walk plus the record spill 88 bytes).
 #define SHIM_TRACE_HIT_THREADS 128
 __global__ void __launch_bounds__(SHIM_TRACE_HIT_THREADS, 3) trace_hit_kernel(SceneView sv, const float* rays, long long n, float t_min, float t_max,
                                                         uint64_t seed, f4* out, unsigned long long* counters) {
-    uint32_t nodes = 0, prims = 0;
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const float* q = rays + i * 7;
-        Ray r; r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
-        Rng rng;
-        rng_init(rng, (uint32_t)i, 0, seed);
-        rng_key(rng, 0, STAGE_INTERSECT);
-        TraceCounters tc; tc.nodes = 0; tc.prims = 0; tc.hrpp_tp = 0; tc.hrpp_fp = 0; tc.hrpp_none = 0;
-        Hit h = counters ? closest_hit<true>(sv, r, t_min, t_max, rng, &tc)
-                         : (sv.qnodes ? closest_hit<false, false, true, true>(sv, r, t_min, t_max, rng, &tc) : closest_hit<false>(sv, r, t_min, t_max, rng, &tc));
-        nodes += tc.nodes; prims += tc.prims;
-        f4 w0, w1, w2;
-        hit_record_words(sv, r, h, w0, w1, w2);
-        out[3 * i] = w0;
-        out[3 * i + 1] = w1;
-        out[3 * i + 2] = w2;
-    }
-    if (counters) {
-        atomicAdd(counters + 1, (unsigned long long)nodes);
-        atomicAdd(counters + 2, (unsigned long long)prims);
-    }
+    trace_batch<false>(sv, rays, n, t_min, t_max, seed, counters, StoreRecord{out});
 }
 
-// Occlusion (any hit) for a batch of rays: the rays, node layouts and Philox keying of trace_closest_kernel, the walk
-// ending at the first accepted hit (closest_hit<..., ANY = true>).  occluded[i] = 1 exactly where trace_closest_kernel
-// reports prim_id >= 0.  256-thread blocks, two per SM: 128 registers and no spills (with __launch_bounds__(256) alone
-// ptxas also settles on 128 registers but spills 16 bytes, as trace_closest_kernel does).
+// Occlusion (any hit) for a batch of rays: occluded[i] = 1 exactly where trace_closest_kernel reports prim_id >= 0.
+// 256-thread blocks, two per SM: 128 registers and no spills (with __launch_bounds__(256) alone ptxas also settles on
+// 128 registers but spills 16 bytes, as trace_closest_kernel does).
 #define SHIM_TRACE_OCCLUDED_THREADS 256
 __global__ void __launch_bounds__(SHIM_TRACE_OCCLUDED_THREADS, 2) trace_occluded_kernel(SceneView sv, const float* rays, long long n, float t_min,
                                                                                      float t_max, uint64_t seed, uint8_t* occluded,
                                                                                      unsigned long long* counters) {
-    uint32_t nodes = 0, prims = 0;
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const float* q = rays + i * 7;
-        Ray r; r.o = mk3(q[0], q[1], q[2]); r.d = mk3(q[3], q[4], q[5]); r.time = q[6];
-        Rng rng;
-        rng_init(rng, (uint32_t)i, 0, seed);
-        rng_key(rng, 0, STAGE_INTERSECT);
-        TraceCounters tc; tc.nodes = 0; tc.prims = 0; tc.hrpp_tp = 0; tc.hrpp_fp = 0; tc.hrpp_none = 0;
-        Hit h = counters ? closest_hit<true, false, true, false, true>(sv, r, t_min, t_max, rng, &tc)
-                         : (sv.qnodes ? closest_hit<false, false, true, true, true>(sv, r, t_min, t_max, rng, &tc)
-                                      : closest_hit<false, false, true, false, true>(sv, r, t_min, t_max, rng, &tc));
-        nodes += tc.nodes; prims += tc.prims;
-        occluded[i] = h.obj >= 0 ? 1 : 0;
-    }
-    if (counters) {
-        atomicAdd(counters + 1, (unsigned long long)nodes);
-        atomicAdd(counters + 2, (unsigned long long)prims);
-    }
+    trace_batch<true>(sv, rays, n, t_min, t_max, seed, counters, StoreOccluded{occluded});
 }
 
 }  // namespace shim

@@ -63,6 +63,8 @@ def oracle_lib():
         lib.orc_texture_value.argtypes = [_P, _I, _F, _F, _P, _P]
         lib.orc_trace_closest.restype = _I
         lib.orc_trace_closest.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _I, _P, _P, _P]
+        lib.orc_trace_record.restype = _I
+        lib.orc_trace_record.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P]
         lib.orc_render.restype = _I
         lib.orc_render.argtypes = [_P, _P, C.POINTER(OrcRenderParams), _P, C.POINTER(OrcStats)]
         lib.orc_sample_radiance.restype = _I
@@ -98,12 +100,18 @@ def hostsim_lib():
         lib.hs_trace_closest.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _P, _P, _P]
         lib.hs_trace_closest_q.restype = _I
         lib.hs_trace_closest_q.argtypes = [_P, _P, C.c_int64, _F, _F, _P, _P, _P]
+        lib.hs_trace_hit.restype = _I
+        lib.hs_trace_hit.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _I, _P, _P]
+        lib.hs_trace_occluded.restype = _I
+        lib.hs_trace_occluded.argtypes = [_P, _P, C.c_int64, _F, _F, C.c_uint64, _I, _P, _P]
         lib.hs_qnodes.restype = _I
         lib.hs_qnodes.argtypes = [_P, _P, _I]
         lib.hs_trace_closest_solo.restype = _I
         lib.hs_trace_closest_solo.argtypes = [_P, _P, C.c_int64, _F, _F, _I, _P, _P, _P]
         lib.hs_sample_radiance.restype = _I
         lib.hs_sample_radiance.argtypes = [_P, C.POINTER(Camera), C.POINTER(RenderParams), _P, C.c_int64, _P, _P]
+        lib.hs_render_counts.restype = _I
+        lib.hs_render_counts.argtypes = [_P, C.POINTER(Camera), C.POINTER(RenderParams), _P, C.c_int64, C.c_uint32, _I, _P]
         lib.hs_texture_value.restype = None
         lib.hs_texture_value.argtypes = [_P, _I, _F, _F, _P, _P]
         lib.hs_enable_predictors.restype = _I
@@ -128,6 +136,15 @@ class OracleScene(capi.SceneHandle):
                                         prim.ctypes.data, t.ctypes.data, cnt.ctypes.data)
         assert rc == 0
         return (prim, t, cnt) if counters else (prim, t)
+
+    def trace_hit(self, rays, t_min=0.001, t_max=float("inf"), seed=0, counters=False):
+        """The oracle's HitRecord and hittable id per ray, as a capi.HIT_RECORD_DTYPE array."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 7)
+        n = rays.shape[0]
+        out = np.empty(n, capi.HIT_RECORD_DTYPE); cnt = np.zeros(3, np.uint64)
+        rc = self.lib.orc_trace_record(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, out.ctypes.data, cnt.ctypes.data)
+        assert rc == 0
+        return (out, cnt) if counters else out
 
     def params(self, width, height, spp, max_depth=50, tile=(8, 8), background=(0, 0, 0), seed=0, sample_begin=0,
                sample_count=0, rng_fast=False, iterative=False, threads=0, use_predictors=False, raw_sum=False):
@@ -204,6 +221,29 @@ class HostSimScene(capi.SceneHandle):
         assert nq > 0, "no quantised nodes (not a one-Bvh world, or not representable)"
         return prim, t, cnt, nq
 
+    def trace_hit(self, rays, t_min=0.001, t_max=float("inf"), seed=0, counters=False, quantised=False):
+        """trace_hit_kernel's arithmetic ray by ray (capi.HIT_RECORD_DTYPE array); ``quantised``: the one Bvh object
+        walked on its quantised nodes, as the kernel does for a scene that has them."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 7)
+        n = rays.shape[0]
+        out = np.empty(n, capi.HIT_RECORD_DTYPE); cnt = np.zeros(3, np.uint64)
+        rc = self.lib.hs_trace_hit(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, 1 if quantised else 0, out.ctypes.data,
+                                   cnt.ctypes.data)
+        assert rc == 0, "no quantised nodes (not a one-Bvh world)"
+        return (out, cnt) if counters else out
+
+    def trace_occluded(self, rays, t_min=0.001, t_max=float("inf"), seed=0, counters=False, quantised=False):
+        """trace_occluded_kernel's arithmetic ray by ray (bool per ray); ``quantised``: the one Bvh object walked on its
+        quantised nodes, as the kernel does for a scene that has them."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 7)
+        n = rays.shape[0]
+        out = np.empty(n, np.uint8); cnt = np.zeros(3, np.uint64)
+        rc = self.lib.hs_trace_occluded(self.ptr, rays.ctypes.data, n, t_min, t_max, seed, 1 if quantised else 0, out.ctypes.data,
+                                        cnt.ctypes.data)
+        assert rc == 0, "no quantised nodes (not a one-Bvh world)"
+        occ = out.view(np.bool_)
+        return (occ, cnt) if counters else occ
+
     def enable_predictors(self, log2=16):
         return self.lib.hs_enable_predictors(self.ptr, log2)
 
@@ -219,7 +259,25 @@ class HostSimScene(capi.SceneHandle):
         self.lib.hs_sample_radiance(self.ptr, C.byref(camera), C.byref(p), xys.ctypes.data, len(xys), out.ctypes.data, C.byref(rays))
         return out, rays.value
 
+    def render_counts(self, camera: Camera, p: RenderParams, xys, tail_threshold=65536, generic=False):
+        """(rays, node visits, primitive tests) of a counted render of the samples ``xys`` (n x 3: x, y, sample) with a
+        pool that holds all of them and the endgame threshold ``tail_threshold``; ``generic``: every ray counted as
+        closest_hit counts it."""
+        xys = np.ascontiguousarray(xys, np.int32).reshape(-1, 3)
+        out = np.zeros(3, np.uint64)
+        rc = self.lib.hs_render_counts(self.ptr, C.byref(camera), C.byref(p), xys.ctypes.data, len(xys), tail_threshold,
+                                       1 if generic else 0, out.ctypes.data)
+        assert rc == 0
+        return tuple(int(v) for v in out)
+
 
 def random_xys(width, height, spp, n, seed=0):
     rs = np.random.RandomState(seed)
     return np.stack([rs.randint(0, width, n), rs.randint(0, height, n), rs.randint(0, spp, n)], axis=1).astype(np.int32)
+
+
+def all_samples(width, height, spp, sample_begin=0, sample_count=0):
+    """Every (x, y, sample) of a render (sample_count 0: all spp samples), in no particular order."""
+    count = sample_count if sample_count > 0 else spp
+    y, x, s = np.meshgrid(np.arange(height), np.arange(width), np.arange(sample_begin, sample_begin + count), indexing="ij")
+    return np.stack([x.ravel(), y.ravel(), s.ravel()], axis=1).astype(np.int32)

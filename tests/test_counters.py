@@ -2,7 +2,7 @@
 primitive tests.  bench.py divides node visits and primitive tests by rays to get its instruction budget, so they are
 held to an exact CPU count here.
 
-The reference is tests/records/hostsim_counts.cpp (hs_render_counts): the paths of hs_sample_radiance, every ray counted
+The reference is hs_render_counts in tests/hostsim/hostsim.cpp: the paths of hs_sample_radiance, every ray counted
 as the kernel that traces it in the render counts it.  A counted render walks the exact 64-byte nodes:
   - a world with one Bvh among plain objects and no medium goes through the mesh pipeline (wf_bvh1_list + wf_bvh1_walk):
     one primitive test per list object, the root's two child boxes against the closest list hit as a gate that is not a
@@ -22,7 +22,6 @@ from unittest import mock
 import numpy as np
 import pytest
 
-import counters_support as CS
 import support
 import test_gpu_parity as T
 from raytracinginoneweekendinrust_b200 import api, capi, scenes
@@ -36,7 +35,7 @@ TAIL = 65536                                                               # the
 
 
 def harness(name, reference_tree=False):
-    h = CS.HostSimScene()
+    h = support.HostSimScene()
     h.set_device_bvh(reference_tree)
     info = scenes.build(h, name, seed=1, **T.SMALL.get(name, {}))
     return h, info
@@ -93,7 +92,7 @@ def test_flat_world_counts_in_closed_form(name):
     prim_tests = (rays - NaN rays) x objects, rays from the oracle's integrator."""
     o = support.OracleScene()
     info = scenes.build(o, name, seed=1)
-    h = CS.HostSimScene()
+    h = support.HostSimScene()
     objects = []
     add = h.world_add
     h.world_add = lambda obj: (objects.append(obj), add(obj))[1]
@@ -150,7 +149,7 @@ def test_gpu_counted_render(name):
     np.testing.assert_allclose(img, plain, rtol=2e-5, atol=2e-6)
     ref, so = o.render(cam, o.params(W, H, spp, 50, background=info.background, seed=5))
     assert_image_matches_oracle(name, img, st, ref, so, W, H)
-    assert_counts_match_harness(name, counts(st), h.render_counts(cam, p, CS.all_samples(W, H, spp), TAIL))
+    assert_counts_match_harness(name, counts(st), h.render_counts(cam, p, support.all_samples(W, H, spp), TAIL))
 
 
 @pytest.mark.gpu
@@ -164,7 +163,7 @@ def test_gpu_counted_render_endgame_mid_render(name):
     p = api.make_params(W, H, spp, 50, background=info.background, seed=7, flags=COUNT)
     _, st = g.render(cam, p)
     assert st.iterations > 1 or name == "earth"   # a lone sphere: at most 65 536 paths outlive the camera rays
-    assert_counts_match_harness(name, counts(st), h.render_counts(cam, p, CS.all_samples(W, H, spp), TAIL))
+    assert_counts_match_harness(name, counts(st), h.render_counts(cam, p, support.all_samples(W, H, spp), TAIL))
 
 
 @pytest.mark.gpu
@@ -178,7 +177,7 @@ def test_gpu_counts_do_not_depend_on_how_the_render_runs(name):
     h, _ = harness(name)
     cam = T.CAMERAS[name]
     W, H, spp = 64, 48, 4
-    xys = CS.all_samples(W, H, spp)
+    xys = support.all_samples(W, H, spp)
     p = api.make_params(W, H, spp, 50, background=info.background, seed=5, flags=COUNT)
     small = api.make_params(W, H, spp, 50, background=info.background, seed=5, flags=COUNT, pool_paths=2048)
     _, base = g.render(cam, p)

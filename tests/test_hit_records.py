@@ -1,7 +1,7 @@
 """Hittable::hit with the whole HitRecord (shim_trace_hit): record-level parity with the oracle.
 
-On the CPU the product's device arithmetic (tests/hostsim: closest_hit + reconstruct_hit, as trace_hit_kernel runs
-them) must give the oracle's record bit for bit, every field compared as raw bits.  With -m gpu the CUDA kernel is
+On the CPU the product's device arithmetic (hs_trace_hit in tests/hostsim: trace_hit_kernel's loop and record words)
+must give the oracle's record bit for bit, every field compared as raw bits.  With -m gpu the CUDA kernel is
 compared the same way; there the device acosf / atan2f of the sphere uv and the device logf of a medium's free path
 may differ from glibc by an ulp (stated per test)."""
 import ctypes as C
@@ -9,7 +9,6 @@ import ctypes as C
 import numpy as np
 import pytest
 
-import records_support as R
 import support
 import test_gpu_parity as T
 from fuzz_scenes import build_random_scene, random_rays
@@ -73,7 +72,7 @@ def scene_rays(o, name, info, n_paths=1500, cap=20000, seed=4):
 @pytest.mark.parametrize("name", list(scenes.SCENES))
 def test_device_records_match_oracle_bit_for_bit(name, reference_tree):
     kw = T.SMALL.get(name, {})
-    o, h = R.OracleScene(), R.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     info = scenes.build(o, name, seed=1, **kw)
     h.set_device_bvh(reference_tree)
     scenes.build(h, name, seed=1, **kw)
@@ -100,7 +99,7 @@ def test_device_records_match_oracle_bit_for_bit(name, reference_tree):
 def test_quantised_mesh_walk_gives_the_same_records(name):
     """A mesh among the Cornell rects is queried on its quantised nodes (what the kernel walks for such a scene)."""
     kw = T.SMALL.get(name, {})
-    o, h = R.OracleScene(), R.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     info = scenes.build(o, name, seed=1, **kw)
     scenes.build(h, name, seed=1, **kw)
     rays = scene_rays(o, name, info)
@@ -112,7 +111,7 @@ def test_quantised_mesh_walk_gives_the_same_records(name):
 @pytest.mark.parametrize("reference_tree", [False, True])
 @pytest.mark.parametrize("seed", range(6))
 def test_fuzz_scene_records_match_oracle(seed, reference_tree):
-    o, h = R.OracleScene(), R.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     build_random_scene(o, seed)
     h.set_device_bvh(reference_tree)
     build_random_scene(h, seed)
@@ -162,7 +161,7 @@ def _aimed_rays(centres, per, seed):
 def test_every_record_field_is_covered():
     """Sphere and moving-sphere uv, rect uv, cube sides, the triangle normal, RotateY's mixed-space set_face_normal with
     front_face left as the inner hit set it, Translate's moved point and the medium record, against the oracle."""
-    o, h = R.OracleScene(), R.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     ids, phase, after = _field_scene(o)
     assert _field_scene(h) == (ids, phase, after)
     assert after == phase + 1
@@ -208,7 +207,7 @@ def test_every_record_field_is_covered():
 
 
 def test_miss_record_is_exact():
-    o, h = R.OracleScene(), R.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     for s in (o, h):
         scenes.build(s, "random-spheres", seed=1)
     rays = np.array([[0, 50, 0, 0, 1, 0, 0], [0, 2000, 0, 1, 0.5, 0, 0.5]], np.float32)
@@ -277,16 +276,16 @@ def test_no_cpu_fallback_without_a_device():
 
 # ------------------------------------------------------------------------------------------------ GPU
 def build_pair(name, seed=1):
-    """The product scene and the oracle scene (with orc_trace_hit) of one of scenes.SCENES, at the parity tests' sizes."""
+    """The product scene and the oracle scene (with orc_trace_record) of one of scenes.SCENES, at the parity tests' sizes."""
     g = api.Scene()
     info = scenes.build(g, name, seed=seed, **T.SMALL.get(name, {}))
-    o = R.OracleScene()
+    o = support.OracleScene()
     scenes.build(o, name, seed=seed, **T.SMALL.get(name, {}))
     return g, o, info
 
 
 def _sphere_and_medium_ids(name):
-    k = _Kinds(R.OracleScene())
+    k = _Kinds(support.OracleScene())
     scenes.build(k, name, seed=1, **T.SMALL.get(name, {}))
     return k.spheres, k.media
 

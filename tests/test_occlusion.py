@@ -2,7 +2,7 @@
 
 Its walk is the closest-hit walk cut off at the first accepted hit, so for every ray, seed and interval
 ``occluded == (trace_closest(...).prim_id >= 0)`` bit for bit, with no more node visits or primitive tests.  On the CPU
-the product's device arithmetic (tests/records/hostsim_occluded.cpp: closest_hit<..., ANY = true>) is checked against its
+the product's device arithmetic (hs_trace_occluded in tests/hostsim: closest_hit<..., ANY = true>) is checked against its
 own closest-hit query (exact) and against the oracle's ``prim >= 0``.  With -m gpu the kernel is checked the same way
 against shim_trace_closest (exact, media included: both draw the same device logf) and against the oracle, where media
 scenes may also differ by gate 1b's number of flipped accepts (device logf).
@@ -16,8 +16,6 @@ recorded hit points a and b (origin a, direction b - a, t in [1e-3, 1 - 1e-3]), 
 import numpy as np
 import pytest
 
-import occlusion_support as OS
-import records_support as R
 import support
 import test_gpu_parity as T
 import test_hit_records as HR
@@ -78,7 +76,7 @@ def check_against_closest(h, o, rays, t_min, t_max, seed, what):
 @pytest.mark.parametrize("name", list(scenes.SCENES))
 def test_occluded_is_closest_hit_found(name, reference_tree):
     kw = T.SMALL.get(name, {})
-    o, h = R.OracleScene(), OS.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     info = scenes.build(o, name, seed=1, **kw)
     h.set_device_bvh(reference_tree)
     scenes.build(h, name, seed=1, **kw)
@@ -99,7 +97,7 @@ def test_quantised_mesh_walk(name):
     closest-hit walk on the same nodes (the harness's hs_trace_closest_q; these scenes have no media, so the seed does
     not matter)."""
     kw = T.SMALL.get(name, {})
-    o, h, hq = R.OracleScene(), OS.HostSimScene(), support.HostSimScene()
+    o, h, hq = support.OracleScene(), support.HostSimScene(), support.HostSimScene()
     info = scenes.build(o, name, seed=1, **kw)
     scenes.build(h, name, seed=1, **kw)
     scenes.build(hq, name, seed=1, **kw)
@@ -118,7 +116,7 @@ def test_quantised_mesh_walk(name):
 @pytest.mark.parametrize("reference_tree", [False, True])
 @pytest.mark.parametrize("seed", range(6))
 def test_fuzz_scenes(seed, reference_tree):
-    o, h = R.OracleScene(), OS.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     build_random_scene(o, seed)
     h.set_device_bvh(reference_tree)
     build_random_scene(h, seed)
@@ -136,7 +134,7 @@ def test_interval_ends_at_the_hit(name):
     left out: at a bound equal to the hit's t the closest-hit query itself can answer otherwise than the oracle (one
     showcase ray here), a closest-hit parity question outside this query."""
     kw = T.SMALL.get(name, {})
-    o, h = R.OracleScene(), OS.HostSimScene()
+    o, h = support.OracleScene(), support.HostSimScene()
     info = scenes.build(o, name, seed=1, **kw)
     scenes.build(h, name, seed=1, **kw)
     rays = HR.scene_rays(o, name, info, n_paths=200, cap=2000)
@@ -157,7 +155,7 @@ def test_interval_ends_at_the_hit(name):
 
 
 def test_empty_batch_and_misses():
-    h = OS.HostSimScene()
+    h = support.HostSimScene()
     scenes.build(h, "random-spheres", seed=1)
     rays = np.array([[0, 50, 0, 0, 1, 0, 0], [0, 2000, 0, 1, 0.5, 0, 0.5], [0, 1, -30, 0, 0, 1, 0]], np.float32)
     np.testing.assert_array_equal(h.trace_occluded(rays), [False, False, True])
